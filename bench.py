@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- knot-point Jacobian+Hessian evaluations per second (FP64), BASELINE.json metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE configs[1] -- cartpole swing-up, T=101, B=4096 problems PER
 GPU (weak scaling: each rank owns its own contiguous shard of the global batch, no collective on
@@ -18,6 +18,12 @@ pass over the rank's batch.
   cpu_baseline  the oracle's C twin (no-CSE, "what Symbolics 0.1.x emits") on the host cores.
 
 --impl reference times that C twin itself (the reference needs Julia + Ipopt, absent here).
+
+--dump-outputs DIR writes what the last timed step computed, as the host API would return it (J and H, float64), to
+DIR/jacobian.npy and DIR/hessian.npy: rank 0's rows of a fixed, seeded sample of its problems (under 64 MB). The inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
+
+The run writes nothing into the source tree: a model library it has to compile goes to a temporary directory.
 """
 from __future__ import annotations
 
@@ -26,17 +32,20 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # no __pycache__ in the source tree
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 METRIC = "knot-point Jac+Hessian evals/sec (FP64)"
 UNIT = "knot-evals/s"
+DUMP_BYTES = 60 * 10**6  # --dump-outputs: sampled problems x (J + H) rows, under 64 MB with the .npy headers
 
 
 def _peaks():
@@ -263,6 +272,22 @@ def bench_kkt(torch, n, stream, zp, lp, sp_, peak):
     return res
 
 
+def sample_outputs(torch, nlp) -> dict:
+    """Device copies of J and H of a fixed, seeded sample of the batch's problems (rows in ascending order), enqueued on
+    the current stream: taken right behind the last timed step, before later work overwrites the arrays."""
+    from dto_b200.evaluator import A_H, A_J
+    from dto_b200.sqp import _CudaArray
+    B = nlp.batch
+    k = min(B, DUMP_BYTES // (8 * (nlp.num_jacobian + nlp.num_hessian)))
+    dev = torch.device("cuda", nlp.shard_device(0))
+    rows = torch.as_tensor(np.sort(np.random.default_rng(0).choice(B, size=k, replace=False)), device=dev)
+    out = {}
+    for name, arr, width in (("jacobian", A_J, nlp.num_jacobian), ("hessian", A_H, nlp.num_hessian)):
+        view = torch.as_tensor(_CudaArray(nlp.device_pointer(arr, 0), (B, width)), device=dev)
+        out[name] = view.index_select(0, rows)
+    return out
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -337,6 +362,7 @@ def run_ours(args):
         for i in range(args.steps):
             nlps[i % R].launch(K_JAC_HESS)
         e1.record(stream)
+        dumped = sample_outputs(torch, nlps[(args.steps - 1) % R]) if args.dump_outputs and rank == 0 else None
         barrier()
         ms = e0.elapsed_time(e1)
         n1 = sum(n.launch_count() for n in nlps)
@@ -396,6 +422,11 @@ def run_ours(args):
         kkt["e2e_knot_evals_per_s"] = B_total * T / (kkt["e2e_ms_host_z_lambda_to_host_solution"] * 1e-3)
         kkt["n_gpus"] = world
         kkt["timing"] = "max over ranks"
+
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), t.cpu().numpy())
 
     line = None
     if rank == 0:
@@ -477,8 +508,8 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
-    ap.add_argument("--warmup", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 200; 5 with --impl reference)")
+    ap.add_argument("--warmup", type=int, default=None, help="untimed steps before them (default 10; 1 with --impl reference)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=4096)
     ap.add_argument("--T", type=int, default=101)
@@ -488,14 +519,21 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", dest="no_cpu")
     ap.add_argument("--no-kkt", action="store_true", dest="no_kkt")
     ap.add_argument("--no-solve", action="store_true", dest="no_solve")
+    ap.add_argument("--dump-outputs", default=None, dest="dump_outputs", metavar="DIR",
+                    help="write J and H of the last timed step (sampled problems) as DIR/<name>.npy")
     args = ap.parse_args()
-    if args.impl == "reference":
-        if args.steps == 200:
-            args.steps = 5
-        if args.warmup == 10:
-            args.warmup = 1
-        return run_reference(args)
-    return run_ours(args)
+    reference = args.impl == "reference"
+    if args.steps is None:
+        args.steps = 5 if reference else 200
+    if args.warmup is None:
+        args.warmup = 1 if reference else 10
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if reference and args.dump_outputs:
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
+    with tempfile.TemporaryDirectory(prefix="dto_bench_") as cache:
+        os.environ.setdefault("DTO_CACHE_DIR", cache)
+        return run_reference(args) if reference else run_ours(args)
 
 
 if __name__ == "__main__":

@@ -28,6 +28,9 @@ CODEGEN_VERSION = "9"
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC_DIR = os.path.join(PKG_DIR, "csrc")
 MODEL_DIR = os.path.join(PKG_DIR, "_models")
+# libraries (and cut searches) missing from MODEL_DIR are generated here; DTO_CACHE_DIR points it elsewhere, so that a
+# process that must not write into the source tree (bench.py) still reuses what the build left in MODEL_DIR
+CACHE_DIR = os.environ.get("DTO_CACHE_DIR") or MODEL_DIR
 NVCC = os.environ.get("DTO_NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 
@@ -344,13 +347,15 @@ def _cached_cuts(el: ElementSpec, g, res, L, wrt, fused):
     h.update(repr((el.role, [str(v) for v in el.vars], el.jac_rows, el.jac_cols, el.hess_rows, el.hess_cols)).encode())
     for e in el.evaluate:
         h.update(sp.srepr(e).encode())
-    path = os.path.join(MODEL_DIR, f"cuts_{h.hexdigest()[:16]}.json")
-    if os.path.exists(path):
-        with open(path) as f:
-            d = json.load(f)
-        return d["cuts"], d["stats"]
+    fname = f"cuts_{h.hexdigest()[:16]}.json"
+    for p in (os.path.join(MODEL_DIR, fname), os.path.join(CACHE_DIR, fname)):
+        if os.path.exists(p):
+            with open(p) as f:
+                d = json.load(f)
+            return d["cuts"], d["stats"]
     cuts, st = choose_cuts(g, res, L, wrt, fused, max_evals=max_evals)
-    os.makedirs(MODEL_DIR, exist_ok=True)
+    path = os.path.join(CACHE_DIR, fname)
+    os.makedirs(CACHE_DIR, exist_ok=True)
     with open(path + ".tmp", "w") as f:
         json.dump({"cuts": cuts, "stats": st}, f)
     os.replace(path + ".tmp", path)
@@ -819,9 +824,12 @@ def spec_hash(spec: ModelSpec) -> str:
 
 def build_model(spec: ModelSpec, verbose: bool = False, force: bool = False) -> str:
     """Generate + compile (or reuse) the model library; returns the path of the .so."""
-    os.makedirs(MODEL_DIR, exist_ok=True)
     hsh = spec_hash(spec)
-    base = os.path.join(MODEL_DIR, f"{spec.name}_{hsh}")
+    prebuilt = os.path.join(MODEL_DIR, f"{spec.name}_{hsh}.so")
+    if os.path.exists(prebuilt) and not force:
+        return prebuilt
+    os.makedirs(CACHE_DIR, exist_ok=True)
+    base = os.path.join(CACHE_DIR, f"{spec.name}_{hsh}")
     so, cu = base + ".so", base + ".cu"
     if os.path.exists(so) and not force:
         return so

@@ -425,10 +425,15 @@ class COracle:
 
 def build_c_oracle(solver, name: str, shared_parameters: bool = False, cse: bool = False, opt: str = "-O2",
                    verbose: bool = False) -> COracle:
-    os.makedirs(BUILD_DIR, exist_ok=True)
     src = emit_c(solver, shared_parameters, cse)
     h = hashlib.sha256((src + opt).encode()).hexdigest()[:12]
-    base = os.path.join(BUILD_DIR, f"oracle_{name}_{'cse' if cse else 'nocse'}_{h}")
+    fname = f"oracle_{name}_{'cse' if cse else 'nocse'}_{h}"
+    if os.path.exists(os.path.join(BUILD_DIR, fname + ".so")):
+        return COracle(os.path.join(BUILD_DIR, fname + ".so"))
+    # a process that must not write into the source tree (bench.py) points DTO_CACHE_DIR elsewhere
+    cache = os.environ.get("DTO_CACHE_DIR") or BUILD_DIR
+    os.makedirs(cache, exist_ok=True)
+    base = os.path.join(cache, fname)
     if not os.path.exists(base + ".so"):
         with open(base + ".c", "w") as f:
             f.write(src)
