@@ -36,7 +36,8 @@ class SqpOptions(C.Structure):
         (n, C.c_double) for n in ("tol_constraint", "tol_dual", "dual_reg", "reg_first", "reg_min", "reg_max", "reg_inc_first", "reg_inc",
                                   "reg_dec", "armijo", "merit_margin", "merit_rho", "merit_min", "lm_first", "lm_min", "lm_grow", "lm_shrink",
                                   "lm_grow_below", "lm_zero", "lam_max", "exact_below", "mu_init", "barrier_kappa_eps", "barrier_kappa_mu",
-                                  "barrier_theta_mu", "tau_min", "bound_push", "bound_frac", "kappa_sigma", "tiny_step", "bound_relax")]
+                                  "barrier_theta_mu", "tau_min", "bound_push", "bound_frac", "kappa_sigma", "tiny_step", "bound_relax")] + [
+        ("hessian_approximation", C.c_int32)]
 
 
 _lib = None
@@ -114,7 +115,13 @@ def lib() -> C.CDLL:
         "dto_kernel_smem_bytes": (i64, [vp, C.c_int]),
         "dto_shape_compiled_gather": (C.c_int, [vp]),
         "dto_kkt_analyze": (C.c_int, [vp, i64p, i64p]),
+        "dto_kkt_analyze_ex": (C.c_int, [vp, C.c_int, i64p, i64p]),
+        "dto_hessian_block_count": (i64, [vp]),
+        "dto_hessian_block_structure": (C.c_int, [vp, i64p, i64p]),
         "dto_kkt_create": (C.c_int, [vp, C.c_double, C.c_double, C.POINTER(vp)]),
+        "dto_kkt_create_ex": (C.c_int, [vp, C.c_double, C.c_double, C.c_int, C.POINTER(vp)]),
+        "dto_kkt_set_hessian_blocks": (C.c_int, [vp, vp]),
+        "dto_kkt_get_hessian_blocks": (C.c_int, [vp, vp]),
         "dto_kkt_destroy": (None, [vp]),
         "dto_kkt_dim": (i64, [vp]),
         "dto_kkt_bandwidth": (i64, [vp]),

@@ -820,6 +820,114 @@ __global__ void k_ip_end(const dto_sqp_args a)
     }
 }
 
+
+// =====================================================================================================================
+// Knot-block damped BFGS (hessian_approximation = 1; sqp.py `knot_bfgs_update` states it): H of K is one dense symmetric
+// block per knot over that knot's variables, updated once per iteration right after the callbacks (Nocedal & Wright,
+// Procedure 18.2). A group of W lanes owns one (problem, knot) block, lane i row (and, by symmetry, column) i; W = 16 puts
+// two blocks in a warp. Column i of a block is read and written by lane i, so consecutive lanes touch consecutive doubles.
+// =====================================================================================================================
+template <int W>
+__device__ __forceinline__ double gsum(double v)
+{
+#pragma unroll
+    for (int o = W / 2; o > 0; o >>= 1) v += __shfl_xor_sync(FULL, v, o, W);
+    return v;
+}
+
+template <int W>
+__global__ void __launch_bounds__(128) k_qn_update(const dto_sqp_args a)
+{
+    const int i = threadIdx.x & (W - 1);
+    const int64_t gid = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / W;   // (problem, knot) of this group
+    const bool live = gid < a.B * a.T;
+    const int64_t b = live ? gid / a.T : 0;
+    const int t = live ? (int)(gid - b * a.T) : 0;
+    const int n = live ? a.kdim[t] : 0;
+    const bool own = i < n;
+    const int zc = a.kofs[t] + i;                                  // variable of row i
+    // s_i and y_i = (g + J'lam)_i - (gp + Jp'lam)_i (pinned variables masked out); z, g and J become the previous ones
+    double s = 0.0, y = 0.0;
+    if (own) {
+        const int64_t zi = b * a.N_z + zc;
+        const double f = a.free[zc];
+        const double zn = a.z[zi], zo = a.zp[zi], gn = a.bg[zi], go = a.gp[zi];
+        const double* __restrict__ lam = a.lam + b * a.N_c;
+        const double* __restrict__ Jn = a.bJ + b * a.nnz_J;
+        double* __restrict__ Jo = a.Jp + b * a.nnz_J;
+        double jl = 0.0, jlp = 0.0;
+        const int q1 = a.colptr[zc + 1];
+        for (int q0 = a.colptr[zc]; q0 < q1; q0 += 4) {
+            int sl[4];
+            double vl[4], vn[4], vo[4];
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                const bool in = q0 + u < q1;
+                sl[u] = in ? a.colslot[q0 + u] : 0;
+                vl[u] = in ? lam[a.colrow[q0 + u]] : 0.0;
+            }
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                vn[u] = q0 + u < q1 ? Jn[sl[u]] : 0.0;
+                vo[u] = q0 + u < q1 ? Jo[sl[u]] : 0.0;
+            }
+#pragma unroll
+            for (int u = 0; u < 4; ++u)
+                if (q0 + u < q1) {
+                    jl += vn[u] * vl[u];
+                    jlp += vo[u] * vl[u];
+                    Jo[sl[u]] = vn[u];
+                }
+        }
+        s = (zn - zo) * f;
+        y = ((gn + jl) - (go + jlp)) * f;
+        a.zp[zi] = zn;
+        a.gp[zi] = gn;
+    }
+    if (a.it == 0) return;   // (uniform over the launch) the previous point is the one just stored
+    const double ss = gsum<W>(s * s), sy = gsum<W>(s * y), yy = gsum<W>(y * y);
+    bool ok = live && ss > 1.0e-30 && isfinite(ss) && isfinite(sy) && isfinite(yy);
+    uint8_t* upd = a.qn_updated + b * a.T + t;
+    // the block's first update starts from (y'y / s'y) I instead of the identity
+    const bool scale = ok && !*upd && sy > 0.0;
+    const double sc = yy / sy;
+    double* __restrict__ blk = a.blocks + b * a.nnz_blk + (live ? a.boff[t] : 0);
+    const int nmax = (int)__reduce_max_sync(FULL, (unsigned)n);
+    double bs = 0.0;   // (B s)_i = sum_j B(j, i) s_j, j ascending
+    for (int j0 = 0; j0 < nmax; j0 += 4) {
+        double v[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) v[u] = (own && j0 + u < n && !scale) ? blk[(j0 + u) * n + i] : 0.0;
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int j = j0 + u;
+            const double sj = __shfl_sync(FULL, s, j & (W - 1), W);
+            if (own && j < n) bs += (scale ? (j == i ? sc : 0.0) : v[u]) * sj;
+        }
+    }
+    const double sBs = gsum<W>(s * bs);
+    const double th = sy >= 0.2 * sBs ? 1.0 : 0.8 * sBs / (sBs - sy);
+    const double r = th * y + (1.0 - th) * bs;
+    const double sr = gsum<W>(s * r);
+    ok = ok && isfinite(sBs) && isfinite(sr) && sBs > 0.0 && sr > 0.0;
+    // B <- B - (Bs)(Bs)'/s'Bs + r r'/s'r: lane i writes column i (bitwise symmetric: both triangles form the same products)
+    for (int j0 = 0; j0 < nmax; j0 += 4) {
+        double v[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) v[u] = (ok && own && j0 + u < n && !scale) ? blk[(j0 + u) * n + i] : 0.0;
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int j = j0 + u;
+            const double bsj = __shfl_sync(FULL, bs, j & (W - 1), W), rj = __shfl_sync(FULL, r, j & (W - 1), W);
+            if (ok && own && j < n) {
+                const double old = scale ? (j == i ? sc : 0.0) : v[u];
+                blk[j * n + i] = old - (bsj * bs) / sBs + (rj * r) / sr;
+            }
+        }
+    }
+    if (ok && i == 0) *upd = 1;
+}
+
 template <class K, class... Args>
 int launch_warp_per(K kernel, int64_t n, void* stream, Args... args)
 {
@@ -885,3 +993,15 @@ extern "C" int dto_sqp_k_ip_after_first(const dto_sqp_args* a, void* s) { return
 extern "C" int dto_sqp_k_ip_direction(const dto_sqp_args* a, void* s) { return launch_warp_per(k_ip_direction, a->B, s, *a); }
 extern "C" int dto_sqp_k_ip_ls_round(const dto_sqp_args* a, int32_t round, void* s) { return launch_warp_per(k_ip_ls_round, a->B, s, *a, round); }
 extern "C" int dto_sqp_k_ip_end(const dto_sqp_args* a, void* s) { return launch_warp_per(k_ip_end, a->B, s, *a); }
+extern "C" int dto_sqp_k_qn_update(const dto_sqp_args* a, void* s)
+{
+    const int64_t threads = a->B * a->T * a->qn_W;
+    if (threads <= 0) return 0;
+    const unsigned grid = (unsigned)((threads + 127) / 128);
+    if (a->qn_W == 16)
+        k_qn_update<16><<<grid, 128, 0, (cudaStream_t)s>>>(*a);
+    else
+        k_qn_update<32><<<grid, 128, 0, (cudaStream_t)s>>>(*a);
+    const cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : -(int)e;
+}

@@ -84,6 +84,16 @@ typedef struct dto_sqp_args {
     double *mu, *mu_next, *amax, *a_z, *fbar;   /* [B] barrier parameter, step limits, barrier value at z      */
     double* diag;                          /* [B][dim] the diagonal the factor kernel adds to K                 */
     double* bg_w;                          /* = bg, writable (the barrier gradient is added to g)               */
+    /* knot-block damped BFGS (hessian_approximation = 1): block t of a problem covers z[kofs[t], kofs[t] + kdim[t]) and is a
+     * dense row-major kdim[t]^2 matrix at offset boff[t] of the problem's nnz_blk block values */
+    int32_t T, qn_W;                       /* knots; lanes per block (16: two blocks per warp, or 32)           */
+    int32_t nnz_blk, nnz_J;
+    const int32_t *kofs, *kdim, *boff;     /* [T]                                                               */
+    double* blocks;                        /* [B][nnz_blk] the KKT handle's blocks (H of K)                     */
+    const double* bJ;                      /* [B][nnz_J] Jacobian of the callbacks                              */
+    const int32_t *colptr, *colslot, *colrow;   /* the KKT handle's Jacobian-by-column tables (J'lam, rows ascending) */
+    double *zp, *gp, *Jp;                  /* z, g, J of the previous iteration                                */
+    uint8_t* qn_updated;                   /* [B][T] 1 once a block has taken an update (the first one is scaled) */
 } dto_sqp_args;
 
 /* each returns 0 or -(cudaError_t) */
@@ -111,6 +121,8 @@ int dto_sqp_k_ip_end(const dto_sqp_args* a, void* stream);
 int dto_sqp_k_pred_ladder(const dto_sqp_args* a, int32_t count, int32_t m, void* stream);
 /* after the first check: a predicted problem that did turn out bad takes the first working candidate of the second set */
 int dto_sqp_k_pred_pick(const dto_sqp_args* a, int32_t count, int32_t m, void* stream);
+/* knot-block damped BFGS: update every block from s = z - zp, y = (g + J'lam) - (gp + Jp'lam), then zp, gp, Jp = z, g, J */
+int dto_sqp_k_qn_update(const dto_sqp_args* a, void* stream);
 /* slot k * R + j (k-th entry of oidx, j < R) <- z + alpha 2^-j dz and the problem's parameters */
 int dto_sqp_k_multi_trial(const dto_sqp_args* a, int32_t count, int32_t R, void* stream);
 /* per open problem: the first j whose trial passes the Armijo test is taken, as R sequential rounds would */

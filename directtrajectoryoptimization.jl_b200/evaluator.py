@@ -126,6 +126,16 @@ class BatchedNLPData:
                                                                c.ctypes.data_as(C.POINTER(C.c_int64))))
         return r, c
 
+    def hessian_block_structure(self):
+        """(rows, cols), 1-based, sorted: every entry of one dense block per knot over that knot's variables [x_t; u_t]
+        (the last knot: x_T). The H of a KKT system in knot-blocks mode, e.g. the solver's BFGS approximation."""
+        n = int(_lib.lib().dto_hessian_block_count(self.shape))
+        r = np.empty(n, dtype=np.int64)
+        c = np.empty(n, dtype=np.int64)
+        _lib.check(_lib.lib().dto_hessian_block_structure(self.shape, r.ctypes.data_as(C.POINTER(C.c_int64)),
+                                                          c.ctypes.data_as(C.POINTER(C.c_int64))))
+        return r, c
+
     def jacobian_structure(self):
         """MOI.jacobian_structure (src/moi.jl:124): list of 1-based (row, col)."""
         r, c = self.jacobian_structure_arrays()
@@ -432,7 +442,9 @@ class Solver:
             clo, cup = self.nlp.constraint_bounds
             pinned = np.isfinite(lo) & (lo == up)
             rows_ok = bool(np.all((clo == cup) | (np.isneginf(clo) & (cup == 0.0))))      # equalities and c(z) <= 0 rows
-            ok = self.nlp.hessian_lagrangian and rows_ok        # (several devices: one native solve per device, side by side)
+            # a problem without Hessians reaches the native solver when its knot-block BFGS mode is asked for
+            qn = (options or {}).get("hessian_approximation", "exact") == "knot-bfgs"
+            ok = (self.nlp.hessian_lagrangian or qn) and rows_ok        # (several devices: one native solve per device, side by side)
             # (bounds on variables (Bound(action_lower = ..., ...)) and inequality rows (Constraint(...; indices_inequality)): the
             # interior-point mode, in both arms)
             method = ("sqp" if record_iterates else "native") if ok else "broker"
@@ -469,6 +481,7 @@ class Solver:
             return res
         from .driver import solve_batch
         opts = dict(options or {})
+        opts.pop("hessian_approximation", None)         # (SciPy's trust-constr keeps its own quasi-Newton approximation)
         ref_opts = self.options if isinstance(self.options, dict) else {}
         if "tol" in ref_opts and "gtol" not in opts:        # Options.tol (src/options.jl:7)
             opts["gtol"] = float(ref_opts["tol"])

@@ -20,25 +20,42 @@ from . import _lib
 from .evaluator import BatchedNLPData, _out, _p
 
 
-def analyze(nlp: BatchedNLPData):
+HESSIAN = {"exact": 0, "knot-blocks": 1}   # DTO_KKT_HESSIAN_EXACT, DTO_KKT_HESSIAN_KNOT_BLOCKS
+
+
+def _hessian_mode(hessian: str) -> int:
+    if hessian not in HESSIAN:
+        raise ValueError(f"hessian={hessian!r}: expected one of {sorted(HESSIAN)}")
+    return HESSIAN[hessian]
+
+
+def analyze(nlp: BatchedNLPData, hessian: str = "exact"):
     """Host-only symbolic phase: (perm, bandwidth). perm[p] is the 1-based index (variables first,
-    then constraint rows) placed at position p of the banded ordering."""
+    then constraint rows) placed at position p of the banded ordering. hessian="knot-blocks": the H block
+    of K is one dense block per knot (nlp.hessian_block_structure()) instead of the Hessian's structure."""
     n = nlp.num_variables + nlp.num_constraint
     perm = np.empty(n, dtype=np.int64)
     bw = C.c_int64()
-    _lib.check(_lib.lib().dto_kkt_analyze(nlp.shape, perm.ctypes.data_as(C.POINTER(C.c_int64)), C.byref(bw)))
+    _lib.check(_lib.lib().dto_kkt_analyze_ex(nlp.shape, _hessian_mode(hessian), perm.ctypes.data_as(C.POINTER(C.c_int64)), C.byref(bw)))
     return perm, int(bw.value)
 
 
 class KKTSystem:
-    """K sol = h for all problems of `nlp` (pendulum.jl:138-211 batched)."""
+    """K sol = h for all problems of `nlp` (pendulum.jl:138-211 batched).
 
-    def __init__(self, nlp: BatchedNLPData, primal_reg: float = 1.0e-5, dual_reg: float = 1.0e-5):
+    hessian="knot-blocks": H is not the callbacks' Hessian but one dense symmetric block per knot owned by this
+    object (the identity at first; set_hessian_blocks / hessian_blocks, shape [B, nnz_blk] in the order of
+    nlp.hessian_block_structure()); the callbacks then run without a Hessian pass, so a problem built without
+    evaluate_hessian works."""
+
+    def __init__(self, nlp: BatchedNLPData, primal_reg: float = 1.0e-5, dual_reg: float = 1.0e-5, hessian: str = "exact"):
         L = _lib.lib()
         self.nlp = nlp
+        self.hessian = hessian
         h = C.c_void_p()
-        _lib.check(L.dto_kkt_create(nlp.handle, float(primal_reg), float(dual_reg), C.byref(h)))
+        _lib.check(L.dto_kkt_create_ex(nlp.handle, float(primal_reg), float(dual_reg), _hessian_mode(hessian), C.byref(h)))
         self._h = h
+        self.num_blocks = int(L.dto_hessian_block_count(nlp.shape)) if hessian == "knot-blocks" else 0
         self.dim = int(L.dto_kkt_dim(h))
         self.bandwidth = int(L.dto_kkt_bandwidth(h))
         self.row_width = int(L.dto_kkt_row_width(h))
@@ -143,6 +160,18 @@ class KKTSystem:
             idx = np.arange(q, self.dim)
             Lm[idx, idx - q] = band[q:, q]
         return Lm, D
+
+    def set_hessian_blocks(self, blocks) -> None:
+        """knot-blocks mode: the blocks of every problem, [B, nnz_blk] (host -> device)."""
+        from .evaluator import _f64
+        v = _f64(blocks, (self.nlp.batch, self.num_blocks), "blocks")
+        _lib.check(_lib.lib().dto_kkt_set_hessian_blocks(self._h, _p(v)))
+
+    def hessian_blocks(self) -> np.ndarray:
+        """knot-blocks mode: the blocks of every problem, [B, nnz_blk] (device -> host)."""
+        out = np.empty((self.nlp.batch, self.num_blocks))
+        _lib.check(_lib.lib().dto_kkt_get_hessian_blocks(self._h, _p(out)))
+        return out
 
     def device_pointer(self, which: int, shard: int = 0) -> int:
         p = _lib.lib().dto_kkt_device_pointer(self._h, int(which), int(shard))

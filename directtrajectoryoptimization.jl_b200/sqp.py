@@ -44,6 +44,15 @@ from dataclasses import dataclass
 from typing import Optional
 
 
+class HessianApproximation(str):
+    """"exact" or "knot-bfgs": a str whose float() is its dto_sqp_options.hessian_approximation code"""
+
+    CODES = {"exact": 0, "knot-bfgs": 1}
+
+    def __float__(self):
+        return float(self.CODES[str(self)])
+
+
 @dataclass
 class SQPOptions:
     max_iter: int = 200
@@ -92,6 +101,9 @@ class SQPOptions:
     tiny_step: float = 1.0e-6          # relative step size under which the full (fraction-to-the-boundary) step is taken untested
     bound_relax: float = 10.0          # fallback of `solve_bounded` for problems the direct solve leaves unconverged: two-sided bounds
                                        #   widened about their midpoint by this factor, solved, then the true bounds warm-started (<= 1: off)
+    hessian_approximation: str = HessianApproximation("exact")   # "knot-bfgs": H is one dense block per knot, updated by damped BFGS (`knot_bfgs_update`) --
+                                       #   for problems built without Hessians (the reference's default evaluate_hessian = false);
+                                       #   the native arm only. exact_below does not apply (H is always the blocks)
 
 
 class SQPResult:
@@ -378,6 +390,39 @@ def solve(be, z0, lam0=None, options: Optional[SQPOptions] = None, record: bool 
     return SQPResult(out["z"], out["lam"], out["iters"], out["done"], out["cv"], out["dr"], out["f"], history, backend=be)
 
 
+def knot_bfgs_update(xp, blocks, s, y, free, first):
+    """One damped BFGS update (Nocedal & Wright, Procedure 18.2) of M dense symmetric n x n blocks -- the knot blocks of the
+    "knot-bfgs" Hessian approximation, one per (problem, knot); dto_sqp.cu `k_qn_update` is its native form.
+    blocks [M, n, n]; s = z - z_prev and y = (g + J'lam) - (g_prev + J_prev'lam) (the same multipliers in both terms; bound
+    multipliers left out) over the block's variables, [M, n]; free [n] or [M, n]: 0 masks pinned variables out of s and y;
+    first [M] bool: the block has taken no update yet. Returns (blocks, first).
+      skipped (block unchanged) when s's = 0 to 1e-30 (a problem that did not move), a quantity is not finite, or s'Bs or
+      s'r is not positive; on a block's first update with s'y > 0, B is first scaled to (y'y / s'y) I;
+      theta = 1 if s'y >= 0.2 s'Bs else 0.8 s'Bs / (s'Bs - s'y),  r = theta y + (1 - theta) Bs,
+      B <- B - (Bs)(Bs)'/s'Bs + r r'/s'r   (so B+ s = r, and B stays symmetric positive definite)."""
+    s = s * free
+    y = y * free
+    ss, sy, yy = xp.sum_rows(s * s), xp.sum_rows(s * y), xp.sum_rows(y * y)
+    fin = lambda v: xp.finite_rows(v[:, None])  # noqa: E731
+    ok = (ss > 1.0e-30) & fin(ss) & fin(sy) & fin(yy)
+    M, n = int(s.shape[0]), int(s.shape[1])
+    scale = ok & first & (sy > 0.0)
+    sc = yy / xp.where(scale, sy, xp.ones((M,)))
+    eye = xp.eye(n)
+    B0 = xp.where(scale[:, None, None], sc[:, None, None] * eye[None, :, :], blocks)
+    Bs = xp.sum_rows3(B0 * s[:, :, None])             # (B s)_i = sum_j B(j, i) s_j
+    sBs = xp.sum_rows(s * Bs)
+    low = sy < 0.2 * sBs
+    theta = xp.where(low, 0.8 * sBs / xp.where(low, sBs - sy, xp.ones((M,))), xp.ones((M,)))
+    r = theta[:, None] * y + (1.0 - theta)[:, None] * Bs
+    sr = xp.sum_rows(s * r)
+    ok = ok & fin(sBs) & fin(sr) & (sBs > 0.0) & (sr > 0.0)
+    one = xp.ones((M,))
+    dBs, dsr = xp.where(ok, sBs, one), xp.where(ok, sr, one)
+    Bn = B0 - (Bs[:, :, None] * Bs[:, None, :]) / dBs[:, None, None] + (r[:, :, None] * r[:, None, :]) / dsr[:, None, None]
+    return xp.where(ok[:, None, None], Bn, blocks), first & ~ok
+
+
 def bound_arrays(lo, up, options: Optional[SQPOptions] = None, clo=None, cup=None, scale: float = 1.0):
     """numpy: primal_bounds (src/data.jl:123-133) -> what `solve` needs. Returns (fixed, bounds): `fixed` = variables pinned
     by lo == up; `bounds` = None when no other finite bound exists, else dict(hasL, hasU, lo, up, pushL, pushU) with 0/1
@@ -525,6 +570,13 @@ class _XP:
     def to_numpy(self, a):
         return a.detach().cpu().numpy().copy() if self.is_torch else self.m.array(a, copy=True)
 
+    def eye(self, n):
+        return self.m.eye(n, **self._kw())
+
+    def sum_rows3(self, a):
+        """[M, j, i] -> [M, i]: sum over j"""
+        return a.sum(dim=1) if self.is_torch else a.sum(axis=1)
+
 
 # --------------------------------------------------------------------------------------- device backend
 class _CudaArray:
@@ -547,6 +599,8 @@ class DeviceBackend:
         from .kkt import KKTSystem
         if nlp.num_shards != 1:
             raise ValueError("DeviceBackend drives one shard; create one batch per device")
+        if options is not None and options.hessian_approximation != "exact":
+            raise ValueError(f"hessian_approximation={options.hessian_approximation!r} is a mode of the native solver (method='native')")
         self.nlp = nlp
         self.torch = torch
         dev = torch.device("cuda", nlp.shard_device(0))
@@ -785,8 +839,11 @@ def solve_native(nlp, z0, lam0=None, options: Optional[SQPOptions] = None) -> SQ
     L = _lib.lib()
     co = _lib.SqpOptions()
     L.dto_sqp_default_options(C.byref(co))
+    if o.hessian_approximation not in HessianApproximation.CODES:
+        raise ValueError(f"hessian_approximation={o.hessian_approximation!r}: expected one of {sorted(HessianApproximation.CODES)}")
     for name, _ in _lib.SqpOptions._fields_:
-        setattr(co, name, type(getattr(co, name))(getattr(o, name)))
+        v = HessianApproximation.CODES[o.hessian_approximation] if name == "hessian_approximation" else getattr(o, name)
+        setattr(co, name, type(getattr(co, name))(v))
     B, N_z, N_c = nlp.batch, nlp.num_variables, nlp.num_constraint
     z0 = np.ascontiguousarray(z0, dtype=np.float64)
     if z0.shape != (B, N_z):

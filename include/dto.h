@@ -187,9 +187,29 @@ int64_t dto_kernel_smem_bytes(const dto_shape* s, int kernel_id);
  * 1..N_z, constraint rows N_z+1..N_z+N_c) placed at position p; *bandwidth = half bandwidth of
  * the permuted matrix. Either output may be NULL. */
 int dto_kkt_analyze(const dto_shape* s, int64_t* perm, int64_t* bandwidth);
+/* What the H block of K is. EXACT: the Hessian of the Lagrangian from the callbacks (needs evaluate_hessian). KNOT_BLOCKS: one
+ * dense symmetric block per knot over that knot's variables z[x_t; u_t] (the last knot: x_T), owned by the KKT handle and set
+ * by its caller -- e.g. a quasi-Newton approximation for problems built without Hessians (the reference's evaluate_hessian =
+ * false, which hands Ipopt's limited-memory mode the problem). The blocks are contiguous: block t is a dense row-major
+ * n_t x n_t matrix, n_t = nx_t + nu_t, at offset sum_{s<t} n_s^2 of a problem's nnz_blk = sum_t n_t^2 values. */
+#define DTO_KKT_HESSIAN_EXACT 0
+#define DTO_KKT_HESSIAN_KNOT_BLOCKS 1
+/* nnz_blk, and the (row, col) of every block entry, 1-based, sorted (both triangles, like dto_hessian_lagrangian_structure) */
+int64_t dto_hessian_block_count(const dto_shape* s);
+int dto_hessian_block_structure(const dto_shape* s, int64_t* rows, int64_t* cols);
+/* dto_kkt_analyze for either Hessian structure; KNOT_BLOCKS fails with DTO_ERR_UNSUPPORTED when a knot has more than 32
+ * variables or the ordered half bandwidth exceeds 31 */
+int dto_kkt_analyze_ex(const dto_shape* s, int hessian, int64_t* perm, int64_t* bandwidth);
 /* fails with DTO_ERR_UNSUPPORTED when the ordered half bandwidth exceeds 31. The handle borrows the
  * batch: destroy it BEFORE dto_batch_destroy(b); like the batch it is used from one host thread at a time. */
 int dto_kkt_create(dto_batch* b, double primal_reg, double dual_reg, dto_kkt** out);
+/* dto_kkt_create(...) = dto_kkt_create_ex(..., DTO_KKT_HESSIAN_EXACT, ...). With KNOT_BLOCKS the handle owns the blocks
+ * [B][nnz_blk] (the identity at creation), the shape needs no Hessian, and every callback pass below evaluates the gradient,
+ * the constraints and the Jacobian only (no Hessian pass). */
+int dto_kkt_create_ex(dto_batch* b, double primal_reg, double dual_reg, int hessian, dto_kkt** out);
+/* host <-> device copies of the knot blocks, [B][nnz_blk] (KNOT_BLOCKS handles only) */
+int dto_kkt_set_hessian_blocks(dto_kkt* k, const double* blocks);
+int dto_kkt_get_hessian_blocks(dto_kkt* k, double* blocks);
 void dto_kkt_destroy(dto_kkt* k);
 int64_t dto_kkt_dim(const dto_kkt* k);                       /* N_z + N_c                              */
 int64_t dto_kkt_bandwidth(const dto_kkt* k);                 /* half bandwidth after ordering          */
@@ -240,7 +260,8 @@ int dto_kkt_factor(dto_kkt* k, int64_t problem, double* Lband, double* D);
  * kernels to per-problem mode: the caller writes it on the device), 4 negative-pivot counts [shard size] int32,
  * 5 a per-problem diagonal [shard size][dim] (natural order: variables, then constraint rows) ADDED to K from then on (zero
  * at first: the barrier terms of an interior-point solver -- z_L / (x - l) + z_U / (u - x) on variables with Bound(...),
- * src/bounds.jl; -t_i / lambda_i on inequality rows, Constraint(...; indices_inequality), src/constraints.jl) */
+ * src/bounds.jl; -t_i / lambda_i on inequality rows, Constraint(...; indices_inequality), src/constraints.jl), 6 the knot blocks
+ * [shard size][nnz_blk] (KNOT_BLOCKS handles only) */
 void* dto_kkt_device_pointer(dto_kkt* k, int which, int shard);
 
 /* ---- batched solver: the caller of the callback path (SURVEY 8f N1) ----
@@ -274,6 +295,9 @@ typedef struct dto_sqp_options {
     double tiny_step;        /* relative step size under which a step is taken without the merit test */
     double bound_relax;      /* > 1: problems left unconverged are solved again with two-sided bounds widened by this factor, then
                                 the true bounds warm-started from there (<= 1: no such fallback) */
+    int32_t hessian_approximation;   /* 0: the exact Hessian of the Lagrangian (needs evaluate_hessian); 1: knot-block damped BFGS
+                                        (no Hessian needed: one dense block per knot, updated once per iteration from the change of
+                                        the Lagrangian's gradient; Nocedal & Wright, Procedure 18.2) */
 } dto_sqp_options;
 void dto_sqp_default_options(dto_sqp_options* o);
 /* Solves every problem of a one-shard batch (several devices: one batch and one host thread per device) from z0 [B][N_z] (lambda0 [B][N_c] or NULL = 0). lower / upper [N_z] or

@@ -386,7 +386,7 @@ function DTO.initialize_controls!(solver::Solver, actions; problem::Int=0)
 end
 
 # ---------------------------------------------------------------- batched solve (dto_sqp_solve, include/dto.h)
-"dto_sqp_options: same fields, same order (4 Int32 then 31 Float64)"
+"dto_sqp_options: same fields, same order (4 Int32, then 31 Float64, then 1 Int32)"
 Base.@kwdef struct SQPOptions
     max_iter::Int32 = 200;  max_refactor::Int32 = 14;  max_backtrack::Int32 = 10;  soc::Int32 = 1
     tol_constraint::Float64 = 1.0e-8;  tol_dual::Float64 = 1.0e-6;  dual_reg::Float64 = 1.0e-9
@@ -399,6 +399,7 @@ Base.@kwdef struct SQPOptions
     mu_init::Float64 = 0.1;  barrier_kappa_eps::Float64 = 10.0;  barrier_kappa_mu::Float64 = 0.2;  barrier_theta_mu::Float64 = 1.5
     tau_min::Float64 = 0.99;  bound_push::Float64 = 1.0e-2;  bound_frac::Float64 = 1.0e-2;  kappa_sigma::Float64 = 1.0e10
     tiny_step::Float64 = 1.0e-6;  bound_relax::Float64 = 10.0
+    hessian_approximation::Int32 = 0      # 0 exact Hessian, 1 knot-block damped BFGS (problems built with evaluate_hessian = false)
 end
 
 """
@@ -429,10 +430,14 @@ function solve_batch(nlp::BatchedNLPData, z0::Matrix{Float64}; lower=nothing, up
     (z=z, lambda=lam, iterations=Int.(its), converged=conv .!= 0, constraint_violation=cv, dual_residual=dr, objective=f, stats=stats)
 end
 
-function DTO.solve!(solver::Solver)
+# hessian_approximation = :knot_bfgs solves a batch built without Hessians (the reference's default evaluate_hessian = false,
+# which puts Ipopt in its limited-memory quasi-Newton mode) with the native solver's knot-block damped BFGS
+function DTO.solve!(solver::Solver; hessian_approximation::Symbol=:exact)
     size(solver.z0, 2) == 1 && return MOI.optimize!(solver.optimizer)
+    hessian_approximation in (:exact, :knot_bfgs) || throw(ArgumentError("hessian_approximation must be :exact or :knot_bfgs"))
     max_iter = Int32(get(solver.optimizer.options, "max_iter", 200))               # Options.max_iter (src/options.jl:9)
-    solve_batch(solver.nlp, solver.z0; lower=solver.lower, upper=solver.upper, options=SQPOptions(max_iter=max_iter))
+    options = SQPOptions(max_iter=max_iter, hessian_approximation=Int32(hessian_approximation === :knot_bfgs))
+    solve_batch(solver.nlp, solver.z0; lower=solver.lower, upper=solver.upper, options=options)
 end
 "the last z any callback was handed (the reference returns its internal per-knot buffers, src/solver.jl:41-43)"
 function DTO.get_trajectory(solver::Solver; problem::Int=1)
