@@ -47,15 +47,26 @@ def _deriv_mode() -> str:
     return m
 
 
+# DTO_TUNE keys: the accepted values, the default first. ws / persist: use the warp-specialised / persistent kernel
+# where the shape allows; ws_all: the warp-specialised kernel for the passes without a Hessian too; ws_plan: its
+# precomputed tile plans; ws_helpers: its helper warps; bf: branch-free sin/cos/reciprocal; emit: statement order of
+# the element programs (2: register-pressure-aware list scheduling, 0: DFS post-order)
+TUNE_VALUES = {"ws": (1, 0), "persist": (1, 0), "ws_all": (0, 1), "ws_plan": (1, 0), "ws_helpers": (8, 4), "bf": (1, 0),
+               "emit": (2, 0)}
+
+
 def _tuning() -> Dict[str, int]:
-    """Compile-time kernel tuning (part of the content hash): warps per CTA and the minimum
-    resident CTAs per SM handed to __launch_bounds__ (caps registers per thread).
-    Override with DTO_TUNE="warps=4,min_ctas=3"."""
-    t = {"warps": 2, "min_ctas": 6, "gather_unroll": 4, "emit": 2, "l2_prefetch": 1, "persist": 1, "pwarps": 12, "pctas": 1, "ws": 1, "ws_hreg": 40, "ws_creg": 0, "ws_helpers": 0, "ws_compute": 8, "ws_min_ops": 0, "ws_plan": 1, "ws_all": 0, "bf": 1, "ws_split_gen": 0, "ws_hint": 0, "ws_pdl": 1, "pdl_plain": 1, "live_cap": 56}
+    """Compile-time kernel selection (part of the content hash); override with DTO_TUNE="ws=0,persist=0"."""
+    t = {k: v[0] for k, v in TUNE_VALUES.items()}
     for kv in os.environ.get("DTO_TUNE", "").split(","):
-        if "=" in kv:
-            k, v = kv.split("=")
-            t[k.strip()] = int(v)
+        if not kv.strip():
+            continue
+        k, _, v = kv.partition("=")
+        k = k.strip()
+        if k not in TUNE_VALUES or not v.strip().lstrip("-").isdigit() or int(v) not in TUNE_VALUES[k]:
+            raise ValueError(f"DTO_TUNE: {kv.strip()!r} is not supported; accepted: "
+                             + ", ".join(f"{n}={'|'.join(map(str, vs))}" for n, vs in TUNE_VALUES.items()))
+        t[k] = int(v)
     return t
 
 
@@ -387,17 +398,18 @@ def _emit_element_dag(el: ElementSpec, k: int, out: List[str], stats: dict, cpoo
         stats[f"{pre}_{name}"] = sum(v for kk, v in c.items())
         stats[f"{pre}_{name}_mix"] = c
         chunks.append(f"__device__ __forceinline__ {'double' if ret else 'void'} {pre}_{name}({sig}{extra_sig})\n{{")
-        use_bf = bool(_tuning().get("bf", 0)) and not ret and any(c.get(k_, 0) for k_ in ("sin", "cos", "rcp"))
+        tune = _tuning()
+        use_bf = bool(tune["bf"]) and not ret and any(c.get(k_, 0) for k_ in ("sin", "cos", "rcp"))
         if use_bf:
             # fast path: one basic block; slow path (library sin/cos, IEEE division) only when an argument
             # left the domain of the branch-free functions
             chunks.append("    unsigned dto_bad = 0u;")
-            chunks.extend(emit(g, outputs, load, cpool=cpool, order=_tuning().get("emit", 0), bf=True, live_cap=_tuning().get("live_cap", 56)))
+            chunks.extend(emit(g, outputs, load, cpool=cpool, order=tune["emit"], bf=True))
             chunks.append("    if (__builtin_expect(dto_bad != 0u, 0)) {")
-            chunks.extend(emit(g, outputs, load, indent="        ", prefix="s", cpool=cpool, order=_tuning().get("emit", 0)))
+            chunks.extend(emit(g, outputs, load, indent="        ", prefix="s", cpool=cpool, order=tune["emit"]))
             chunks.append("    }")
         else:
-            chunks.extend(emit(g, outputs, load, cpool=cpool, order=_tuning().get("emit", 0)))
+            chunks.extend(emit(g, outputs, load, cpool=cpool, order=tune["emit"]))
         if ret:
             chunks.append(f"    return {ret};")
         chunks.append("}\n")
@@ -854,23 +866,14 @@ def _build_model_locked(spec: ModelSpec, hsh: str, base: str, so: str, cu: str, 
     if not os.path.exists(NVCC):
         raise RuntimeError(f"nvcc not found at {NVCC}: the CUDA model library cannot be built (no CPU fallback exists)")
     tune = _tuning()
-    # One helper warp per compute warp (16 warps per CTA, 128 registers per thread at launch; setmaxnreg then
-    # gives helpers 40 and compute warps 216). Light models always needed it (a helper's ~300 latency-bound
+    # ws_helpers = 8, one helper warp per compute warp (16 warps per CTA, 128 registers per thread at launch; setmaxnreg
+    # then gives helpers 40 and compute warps 216). Light models always needed it (a helper's ~300 latency-bound
     # integer instructions per tile would bound the kernel); since the hierarchical derivatives cut the
     # FP64 work per knot the heavy models do too: with one helper per TWO compute warps the cartpole compute
     # warps waited 22 % of their time for inputs (profiles/ncu_ws_r02_a.txt), 37.0 -> 33.5 us with 8 helpers.
-    if tune["ws_helpers"] == 0:  # 0 = automatic
-        tune["ws_helpers"] = 8
-    if tune["ws_creg"] == 0:
-        nwarps = tune["ws_helpers"] + tune["ws_compute"]
-        base_regs = min(248, (65536 // (128 * ((nwarps + 3) // 4))) & ~7)   # registers per thread the launch allocates
-        tune["ws_creg"] = min(232, ((nwarps * base_regs - tune["ws_helpers"] * tune["ws_hreg"]) // tune["ws_compute"]) & ~7)
-    cmd = [NVCC, *NVCC_ARCH, f"-DDTO_WARPS={tune['warps']}", f"-DDTO_MIN_CTAS={tune['min_ctas']}",
-           f"-DDTO_GATHER_UNROLL={tune['gather_unroll']}", f"-DDTO_L2_PREFETCH={tune['l2_prefetch']}",
-           f"-DDTO_PERSIST={tune['persist']}", f"-DDTO_PWARPS={tune['pwarps']}", f"-DDTO_PCTAS={tune['pctas']}",
-           f"-DDTO_WS={tune['ws']}", f"-DDTO_WS_HREG={tune['ws_hreg']}", f"-DDTO_WS_CREG={tune['ws_creg']}",
-           f"-DDTO_WS_MIN_OPS={tune['ws_min_ops']}", f"-DDTO_WS_PLAN={tune['ws_plan']}", f"-DDTO_WS_HELPERS={tune['ws_helpers']}", f"-DDTO_WS_COMPUTE={tune['ws_compute']}", f"-DDTO_WS_ALL_MODES={tune['ws_all']}", f"-DDTO_WS_SPLIT_GEN={tune['ws_split_gen']}", f"-DDTO_WS_HINT_NS={tune['ws_hint']}", f"-DDTO_WS_PDL={tune['ws_pdl']}", f"-DDTO_PDL_PLAIN={tune['pdl_plain']}", "-O3", "-std=c++17", "-lineinfo", "--shared", "-Xcompiler", "-fPIC,-fvisibility=hidden", "-Xptxas", "-v",
-           "-I", CSRC_DIR, "-o", so + ".tmp", cu]
+    cmd = [NVCC, *NVCC_ARCH, f"-DDTO_PERSIST={tune['persist']}", f"-DDTO_WS={tune['ws']}", f"-DDTO_WS_PLAN={tune['ws_plan']}",
+           f"-DDTO_WS_HELPERS={tune['ws_helpers']}", f"-DDTO_WS_ALL_MODES={tune['ws_all']}", "-O3", "-std=c++17", "-lineinfo",
+           "--shared", "-Xcompiler", "-fPIC,-fvisibility=hidden", "-Xptxas", "-v", "-I", CSRC_DIR, "-o", so + ".tmp", cu]
     t1 = time.time()
     r = subprocess.run(cmd, capture_output=True, text=True)
     with open(base + ".log", "w") as f:

@@ -26,16 +26,19 @@
 // the slow path, which computes the same records in place.
 #pragma once
 
-#ifndef DTO_WS_COMPUTE
-#define DTO_WS_COMPUTE 8          /* compute warps per CTA: 8 (2 per SM sub-partition) or 12 (3 per sub-partition) */
-#endif
+#define DTO_WS_COMPUTE 8          /* compute warps per CTA (2 per SM sub-partition) */
 #ifndef DTO_WS_HELPERS
-#define DTO_WS_HELPERS 8          /* helper h serves compute warps h, h + HELPERS, ...: COMPUTE must be a multiple */
+#define DTO_WS_HELPERS 8          /* helper h serves compute warps h, h + HELPERS, ...: COMPUTE must be a multiple (DTO_TUNE ws_helpers) */
 #endif
+#define DTO_WS_HREG 40            /* registers per helper-warp thread after setmaxnreg.dec */
 /* registers per thread the launch allocates: 64 K registers per SM over the CTA's threads ROUNDED UP TO 128 (ptxas
  * sizes the pool per group of four warps: 18 warps get 65536/640 = 96, not 112), multiple of 8 */
 #define DTO_WS_WARPS (DTO_WS_COMPUTE + DTO_WS_HELPERS)
 #define DTO_WS_BASE_REGS ((65536 / (128 * ((DTO_WS_WARPS + 3) / 4))) > 255 ? 248 : ((65536 / (128 * ((DTO_WS_WARPS + 3) / 4))) & ~7))
+/* registers per compute-warp thread after setmaxnreg.inc: what the helpers leave of the launch's registers, at most 232
+ * (8 helpers: 216; 4 helpers: 232) */
+#define DTO_WS_CREG_LEFT ((((DTO_WS_WARPS * DTO_WS_BASE_REGS) - DTO_WS_HELPERS * DTO_WS_HREG) / DTO_WS_COMPUTE) & ~7)
+#define DTO_WS_CREG (DTO_WS_CREG_LEFT < 232 ? DTO_WS_CREG_LEFT : 232)
 #define DTO_WS_DESC_DOUBLES 192   /* 3 x int4 per item, 32 items */
 #define DTO_WS_PIECE_DOUBLES 64   /* 1 x int4 per piece, 32 pieces */
 #define DTO_WS_HDR_DOUBLES 2      /* 1 x int4: b0, ... */
@@ -316,15 +319,6 @@ __global__ void __launch_bounds__(128) plan_kernel(const __grid_constant__ dto_l
     P[128 + lane] = piece;
 }
 
-// Option (off by default, DTO_WS_SPLIT_GEN): on light models leave the general-constraint Hessian entries to
-// general_kernel<2> after the knot kernel. Measured slower than the fused single write (car T=201: 306 vs
-// 238 us, profiles/experiments/sweep_r01_y_split_general.jsonl).
-template <class M>
-__host__ __device__ constexpr bool ws_split_general()
-{
-    return DTO_WS_SPLIT_GEN != 0 && M::OPS_FUSED < DTO_WS_MIN_OPS;
-}
-
 // setmaxnreg can only hand out what the launch allocated (12 warps x 168 registers): a split that asks
 // for more makes the compute warps spin in setmaxnreg.inc forever (measured: a hung launch)
 static_assert(DTO_WS_HELPERS <= DTO_WS_COMPUTE && DTO_WS_WARPS <= 32, "at most one helper per compute warp, at most 32 warps");
@@ -347,11 +341,9 @@ __global__ void __launch_bounds__((DTO_WS_COMPUTE + DTO_WS_HELPERS) * 32, 1) kno
     const int T = a.T;
     const int total = (int)(a.B * T);
     const int tiles = (total + OWN - 1) / OWN;
-#if DTO_WS_PDL
     // programmatic dependent launch: the next kernel of the stream may start its CTAs as soon as SMs free up
     // (its own prologue then overlaps this grid's tail); it waits in griddepcontrol.wait before touching data
     asm volatile("griddepcontrol.launch_dependents;");
-#endif
 
     // the knot table lives in shared memory (the launch plan guarantees it fits). Only the slow path (ragged last
     // tile, launches without a plan table) reads it, so nobody waits for it here: one bulk copy, completion on
@@ -383,13 +375,13 @@ __global__ void __launch_bounds__((DTO_WS_COMPUTE + DTO_WS_HELPERS) * 32, 1) kno
     const int4* __restrict__ plan = reinterpret_cast<const int4*>(a.ws_plan);
     const int G4 = ws_gen_int4<MODE>(a);  // int4 of general-constraint records per plan block / stage
 
-    // (DTO_WS_PDL) everything up to here touched only shared memory and launch-constant tables; problem data (z,
-    // lambda, sigma, w, outputs) may still be in use by the previous kernel of the stream until it has completed:
-    // each role executes griddepcontrol.wait right before its first access to problem data
+    // everything up to here touched only shared memory and launch-constant tables; problem data (z, lambda, sigma,
+    // w, outputs) may still be in use by the previous kernel of the stream until it has completed: each role
+    // executes griddepcontrol.wait right before its first access to problem data
     if (warp < DTO_WS_HELPERS) {
         // =============================== helper warp ===============================
         asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(DTO_WS_HREG));
-        bool dep_ok = DTO_WS_PDL == 0;
+        bool dep_ok = false;
         for (int kk = 0;; ++kk) {
             bool any = false;
 #pragma unroll 1
@@ -411,11 +403,7 @@ __global__ void __launch_bounds__((DTO_WS_COMPUTE + DTO_WS_HELPERS) * 32, 1) kno
                 const int od = (kk - 2) & (NOUT - 1), nd = (kk - 2) >> (NOUT - 1);  // output buffer / use count of tile kk-2 (NOUT is 1 or 2)
                 if (have_drain) {
                     // ---- tile kk-2 is complete in output buffer od: issue its stores (piece list of stage st)
-#if defined(DTO_WS_HINT_NS) && DTO_WS_HINT_NS > 0
-                    mbar_wait_hint(bar0 + 16 + od * 8, nd & 1, DTO_WS_HINT_NS);
-#else
                     mbar_wait(bar0 + 16 + od * 8, nd & 1);
-#endif
                     const int4 pd = sdesc[96 + lane];
                     const int b0 = reinterpret_cast<const int*>(sdesc + 128 + G4)[0];
                     int len = pd.w;
@@ -493,9 +481,7 @@ __global__ void __launch_bounds__((DTO_WS_COMPUTE + DTO_WS_HELPERS) * 32, 1) kno
     } else {
         // =============================== compute warp ===============================
         asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(DTO_WS_CREG));
-#if DTO_WS_PDL
         asm volatile("griddepcontrol.wait;" ::: "memory");   // (parameters not staged in shared memory are read from HBM)
-#endif
         const int c = warp - DTO_WS_HELPERS;
         double* __restrict__ smc = dto_smem + kt_doubles + (size_t)c * per_warp;
         const uint32_t bar0 = smem_u32(smc);
@@ -568,7 +554,7 @@ __global__ void __launch_bounds__((DTO_WS_COMPUTE + DTO_WS_HELPERS) * 32, 1) kno
                     double* dst = smc + d2.x + o * out_sz;
                     M::hg_compute_r(hclass, tc, td, ts, pd, v);
                     M::hg_store(hclass, v, dst);
-                    if (a.gen_nhess > 0 && !ws_split_general<M>()) {
+                    if (a.gen_nhess > 0) {
                         // general-constraint entries of this knot's slots: last in the += order (src/moi.jl:112-118)
                         const int b = dsc[128 + G4].x + d2.y, t = d2.z;
                         const int gc = reinterpret_cast<const int*>(dsc + 128 + 32 * DTO_WS_GEN_K)[lane];
@@ -612,7 +598,6 @@ inline int64_t plan_ws(dto_launch_args& b)
     // Hessian pass wins here (FP64-heavy models with 4 helpers + 232-register compute warps, light models
     // with one helper per compute warp: car T=201 256 -> 196 us, pendulum T=11 41 -> 36 us).
     if (!DO_H && !DTO_WS_ALL_MODES) return 0;
-    if (M::OPS_FUSED < DTO_WS_MIN_OPS) return 0;
     if (DO_H && !(M::HG_NCLASS > 0 && b.use_hclass)) return 0;     // table gather: other kernels
     if (M::N_KINDS_MAX >= 255 || M::HG_NCLASS >= 255) return 0;    // descriptor packs kinds in 8 bits
     if (!b.w_flat && b.N_w > 65535) return 0;

@@ -30,58 +30,24 @@
 
 #include "dto_model_abi.h"
 
-#ifndef DTO_WARPS
-#define DTO_WARPS 4
-#endif
-#ifndef DTO_MIN_CTAS
-#define DTO_MIN_CTAS 1
-#endif
-#ifndef DTO_GATHER_UNROLL
-#define DTO_GATHER_UNROLL 8
-#endif
-#ifndef DTO_L2_PREFETCH
-#define DTO_L2_PREFETCH 1
-#endif
+#define DTO_WARPS 2          /* warps per CTA of the plain knot kernel */
+#define DTO_MIN_CTAS 6       /* resident CTAs per SM asked of __launch_bounds__ (caps registers per thread) */
+#define DTO_GATHER_UNROLL 4  /* table-gather records in flight per lane */
+#define DTO_PWARPS 12        /* warps per persistent CTA (upper bound; fewer are launched if shared memory is short) */
+#define DTO_PCTAS 1          /* persistent CTAs per SM */
+#define DTO_KT_SMEM_MAX 384  /* knot-table entries (64 B each) staged in shared memory */
+// Kernel selection, set per model library through DTO_TUNE (codegen._tuning); the tests force each alternative
 #ifndef DTO_PERSIST
 #define DTO_PERSIST 1      /* use the persistent pipeline kernel when the shape allows */
 #endif
-#ifndef DTO_PWARPS
-#define DTO_PWARPS 12      /* warps per persistent CTA (upper bound; fewer are launched if shared memory is short) */
-#endif
-#ifndef DTO_PCTAS
-#define DTO_PCTAS 1        /* persistent CTAs per SM */
-#endif
-#ifndef DTO_KT_SMEM_MAX
-#define DTO_KT_SMEM_MAX 384  /* knot-table entries (64 B each) staged in shared memory */
-#endif
 #ifndef DTO_WS
 #define DTO_WS 1           /* use the warp-specialised kernel when the shape allows */
-#endif
-#ifndef DTO_WS_HREG
-#define DTO_WS_HREG 40     /* registers per helper-warp thread after setmaxnreg.dec */
-#endif
-#ifndef DTO_WS_CREG
-#define DTO_WS_CREG 232    /* registers per compute-warp thread after setmaxnreg.inc (HREG + 2*CREG <= 512) */
-#endif
-#ifndef DTO_WS_PDL
-#define DTO_WS_PDL 0       /* 1: launch the ws kernel with programmatic stream serialization (prologue overlaps the previous kernel's tail) */
-#endif
-#ifndef DTO_PDL_PLAIN
-#define DTO_PDL_PLAIN 1    /* 1: the plain knot kernel is launched with programmatic stream serialization too (it waits for the
-                              previous kernel before touching data, so only launch latency overlaps: cartpole B=4096 gradient
-                              10.3 -> 9.6 us, constraint 18.7 -> 17.1, Jacobian 24.3 -> 21.7) */
 #endif
 #ifndef DTO_WS_PLAN
 #define DTO_WS_PLAN 1      /* precomputed tile-plan table for the ws kernel (0: helpers compute every tile's records) */
 #endif
 #ifndef DTO_WS_ALL_MODES
 #define DTO_WS_ALL_MODES 0 /* 1: ws kernel also for the gradient / residual / Jacobian-only passes */
-#endif
-#ifndef DTO_WS_SPLIT_GEN
-#define DTO_WS_SPLIT_GEN 0 /* 1: ws kernel on light models leaves the general-constraint Hessian to general_kernel<2> (measured slower: car 238 -> 306 us) */
-#endif
-#ifndef DTO_WS_MIN_OPS
-#define DTO_WS_MIN_OPS 0   /* the specialised kernel only for models with at least this many FP64 ops per knot */
 #endif
 #define DTO_SMEM_LIMIT (227 * 1024)
 
@@ -160,10 +126,10 @@ __global__ void __launch_bounds__(DTO_WARPS * 32, DTO_MIN_CTAS) knot_kernel(cons
     constexpr bool DO_J = (MODE & DTO_MODE_J) != 0, DO_H = (MODE & DTO_MODE_H) != 0;
     constexpr bool HALO = DO_H && (M::HESS_HALO != 0);
     constexpr int OWN = HALO ? 31 : 32;
-#if DTO_PDL_PLAIN
+    // launched with programmatic stream serialization: wait for the previous kernel before touching data, so only the
+    // launch latency overlaps (cartpole B=4096 gradient 10.3 -> 9.6 us, constraint 18.7 -> 17.1, Jacobian 24.3 -> 21.7)
     asm volatile("griddepcontrol.launch_dependents;");
     asm volatile("griddepcontrol.wait;" ::: "memory");
-#endif
 
     const int lane = threadIdx.x & 31;
     const int wib = threadIdx.x >> 5;
@@ -388,19 +354,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity)
         asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
                      : "=r"(ok)
                      : "r"(bar), "r"(parity)
-                     : "memory");
-    } while (!ok);
-}
-// the same with a suspend-time hint (ns): the warp sleeps in hardware until the phase completes or the hint
-// expires instead of re-issuing try_wait every ~50 cycles -- for warps whose reaction time does not matter
-// (the ws kernel's helpers), so that their polling does not take issue slots from the compute warps
-__device__ __forceinline__ void mbar_wait_hint(uint32_t bar, uint32_t parity, uint32_t ns)
-{
-    uint32_t ok;
-    do {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ok)
-                     : "r"(bar), "r"(parity), "r"(ns)
                      : "memory");
     } while (!ok);
 }
@@ -892,9 +845,8 @@ inline cudaError_t launch_pdl(K kernel, unsigned grid, unsigned block, size_t sm
 }
 
 template <class M, int MODE>
-inline int launch_knot(const dto_launch_args& a, cudaStream_t st, bool* used_ws)
+inline int launch_knot(const dto_launch_args& a, cudaStream_t st)
 {
-    *used_ws = false;
     constexpr bool HALO = ((MODE & DTO_MODE_H) != 0) && (M::HESS_HALO != 0);
     const long long own = HALO ? 31 : 32;
     const long long total = a.B * (long long)a.T;
@@ -922,16 +874,10 @@ inline int launch_knot(const dto_launch_args& a, cudaStream_t st, bool* used_ws)
             long long ctas = (warps + DTO_WS_COMPUTE - 1) / DTO_WS_COMPUTE;
             if (ctas > sms[dev]) ctas = sms[dev];
             b.ws_plan = ws_get_plan<M, MODE>(b, st);
-#if DTO_WS_PDL
             cudaError_t e = launch_pdl(knot_kernel_ws<M, MODE>, (unsigned)ctas, (DTO_WS_COMPUTE + DTO_WS_HELPERS) * 32, (size_t)wsmem, st, b);
-#else
-            knot_kernel_ws<M, MODE><<<(unsigned)ctas, (DTO_WS_COMPUTE + DTO_WS_HELPERS) * 32, (size_t)wsmem, st>>>(b);
-            cudaError_t e = cudaGetLastError();
-#endif
             if (e != cudaSuccess)
                 fprintf(stderr, "[dto] knot_kernel_ws<mode %d> launch failed: %s (grid %lld, smem %lld)\n", MODE, cudaGetErrorString(e), ctas,
                         (long long)wsmem);
-            *used_ws = true;
             return (int)e;
         }
     }
@@ -973,7 +919,6 @@ inline int launch_knot(const dto_launch_args& a, cudaStream_t st, bool* used_ws)
             return (int)e;
         }
     }
-#if DTO_L2_PREFETCH
     {
         static int resident_warps[16] = {0};  // per device, for the shared-memory size it was computed with
         static int64_t resident_smem[16] = {0};
@@ -992,13 +937,7 @@ inline int launch_knot(const dto_launch_args& a, cudaStream_t st, bool* used_ws)
             b.tiles_in_flight = resident_warps[dev];
         }
     }
-#endif
-#if DTO_PDL_PLAIN
     cudaError_t e = launch_pdl(knot_kernel<M, MODE>, (unsigned)ctas, DTO_WARPS * 32, (size_t)smem, st, b);
-#else
-    knot_kernel<M, MODE><<<(unsigned)ctas, DTO_WARPS * 32, (size_t)smem, st>>>(b);
-    cudaError_t e = cudaGetLastError();
-#endif
     if (e != cudaSuccess)
         fprintf(stderr, "[dto] knot_kernel<mode %d> launch failed: %s (grid %lld, block %d, smem %lld)\n", MODE, cudaGetErrorString(e),
                 ctas, DTO_WARPS * 32, (long long)smem);
@@ -1023,7 +962,6 @@ inline int launch(int kernel_id, const dto_launch_args* pa, void* stream)
     const dto_launch_args& a = *pa;
     cudaStream_t st = (cudaStream_t)stream;
     int e = 0, n = 0;
-    bool ws = false;
     auto general = [&](auto cls, int count) -> int {  // companion kernel over the general-constraint block
         if (count <= 0 || a.B == 0) return 0;
         if ((e = launch_general<M, decltype(cls)::value>(a, st))) return -e;
@@ -1041,28 +979,27 @@ inline int launch(int kernel_id, const dto_launch_args* pa, void* stream)
         e = (int)cudaGetLastError();
         return e ? -e : 1;
     case DTO_K_GRADIENT:
-        e = launch_knot<M, DTO_MODE_G>(a, st, &ws);
+        e = launch_knot<M, DTO_MODE_G>(a, st);
         return e ? -e : 1;
     case DTO_K_CONSTRAINT:
-        if ((e = launch_knot<M, DTO_MODE_C>(a, st, &ws))) return -e;
+        if ((e = launch_knot<M, DTO_MODE_C>(a, st))) return -e;
         ++n;
         if (general(C0{}, a.gen_nrow)) return -e;
         return n;
     case DTO_K_JACOBIAN:
-        if ((e = launch_knot<M, DTO_MODE_J>(a, st, &ws))) return -e;
+        if ((e = launch_knot<M, DTO_MODE_J>(a, st))) return -e;
         ++n;
         if (general(C1{}, a.gen_njac)) return -e;
         return n;
     case DTO_K_HESSIAN:
     case DTO_K_JAC_HESS: {
-        if (kernel_id == DTO_K_HESSIAN) e = launch_knot<M, DTO_MODE_H>(a, st, &ws);
-        else e = launch_knot<M, DTO_MODE_J | DTO_MODE_H>(a, st, &ws);
+        if (kernel_id == DTO_K_HESSIAN) e = launch_knot<M, DTO_MODE_H>(a, st);
+        else e = launch_knot<M, DTO_MODE_J | DTO_MODE_H>(a, st);
         if (e) return -e;
         ++n;
         if (kernel_id == DTO_K_JAC_HESS && general(C1{}, a.gen_njac)) return -e;
-        // general-constraint Hessian: fused into the knot kernel when the compiled gather is in use, unless
-        // the ws kernel runs a light model (ws_split_general)
-        const bool fused = M::HG_NCLASS > 0 && a.use_hclass && !(ws && ws_split_general<M>());
+        // general-constraint Hessian: fused into the knot kernel when the compiled gather is in use
+        const bool fused = M::HG_NCLASS > 0 && a.use_hclass;
         if (!fused && general(C2{}, a.gen_nhess)) return -e;
         return n;
     }

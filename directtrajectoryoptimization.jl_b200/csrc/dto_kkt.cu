@@ -33,10 +33,6 @@
 
 #include "dto_kkt_dev.h"
 
-#ifndef DTO_KKT_PREFETCH
-#define DTO_KKT_PREFETCH 1
-#endif
-
 namespace {
 
 template <int G>
@@ -217,15 +213,13 @@ __device__ __forceinline__ void kkt_backward(const dto_kkt_args& a, unsigned cha
 
 // One problem per group of W lanes (two problems per warp for W = 16). Row block = W rows.
 // BW = compile-time bound on the half bandwidth (<= W - 1).
-// MINB = resident CTAs per SM asked of the compiler: 4 (<= 128 registers, no spills) or 5 (<= 96 registers, a few
-// spilled values; pays off only when the launch has more than 16 warps per SM to offer, i.e. B > ~4700)
 // VIRT = candidate launch (dto_kkt_args::virt): outputs and regularisation indexed by slot. A separate instantiation: as a
 // run-time switch its extra live index cost the default path registers and spills (acrobot, 64 problems: 0.275 vs 0.204 ms)
 // DIAG = a per-problem, per-variable diagonal is added to the Hessian block (dto_kkt_args::diag); separate for the same reason
 // FUSE = the kernel computes the right-hand side itself (dto_kkt_args::fuse_rhs, an option measured slower): its own instantiation too --
 // carrying the code path costs the default kernel 4 % on cartpole (registers)
-template <int W, int BW, int MINB = (W == 16 ? 4 : 2), bool VIRT = false, bool DIAG = false, bool FUSE = false>
-__global__ void __launch_bounds__(128, MINB) kkt_band_kernel(const dto_kkt_args a)
+template <int W, int BW, bool VIRT = false, bool DIAG = false, bool FUSE = false>
+__global__ void __launch_bounds__(128, (W == 16 ? 4 : 2)) kkt_band_kernel(const dto_kkt_args a)
 {
     constexpr int G = W;
     using SM = KktSmem<W, BW>;
@@ -278,7 +272,6 @@ __global__ void __launch_bounds__(128, MINB) kkt_band_kernel(const dto_kkt_args 
     // Static per-row values of the block two ahead (source row of the right-hand side, diagonal shift, pinned flag) are
     // fetched one block early and consumed without branches: a table load followed by a dependent branch or load inside
     // the block loop was a quarter of the time of a launch too small to hide it (profiles/ncu_kkt_latency_r02.txt)
-#if DTO_KKT_PREFETCH
     const double prim = a.preg != nullptr ? a.preg[bo] : a.primal_reg;   // diagonal shift of this slot's variable rows
     int32_t ipn = -1;
     bool fixn = false;
@@ -290,7 +283,6 @@ __global__ void __launch_bounds__(128, MINB) kkt_band_kernel(const dto_kkt_args 
         }
     };
     load_static(2);
-#endif
 
     // ---------------- factor (right-looking) + forward solve ----------------
     // Step j = blk*W + s. v_r = A(r, j) (un-scaled column), l_r = v_r / d_j. The trailing update
@@ -309,7 +301,6 @@ __global__ void __launch_bounds__(128, MINB) kkt_band_kernel(const dto_kkt_args 
                 cp_async8_zfill(stage + w * W + i, sx >= 0 ? (const void*)(bp + sx) : (const void*)Hb, sx >= 0 ? 8 : 0);
             }
             cp_async_commit();
-#if DTO_KKT_PREFETCH
             if (FUSE) {
                 rc = rhs_at(ipn);
             } else {
@@ -320,11 +311,6 @@ __global__ void __launch_bounds__(128, MINB) kkt_band_kernel(const dto_kkt_args 
             if (DIAG && !fixn && ipn >= 0) regc += a.diag[b * a.dim + ipn];
             load_idx(blk + 3);
             load_static(blk + 3);
-#else
-            rc = rhs_at(a.iperm[(size_t)(blk + 2) * W + i]);
-            regc = row_shift<DIAG>(a, (size_t)(blk + 2) * W + i, bo, b);
-            load_idx(blk + 3);
-#endif
         }
         double* LA = Lg + (size_t)blk * W * LW + i;  // + s*LW + (row - j) with immediates
 #pragma unroll
@@ -655,28 +641,26 @@ extern "C" int dto_kkt_launch_rhs(const dto_kkt_args* a, void* stream)
     return e == cudaSuccess ? 1 : -(int)e;
 }
 
-template <int W, int BW, int MINB, bool VIRT, bool DIAG, bool FUSE = false>
+template <int W, int BW, bool VIRT, bool DIAG, bool FUSE = false>
 static cudaError_t launch_band_v(const dto_kkt_args* a, cudaStream_t st)
 {
     const int64_t per_block = 4 * (32 / W);
     // the opt-in is per device and a batch may span several: set it on every launch (a cheap driver call
     // next to a >= 100 us kernel) instead of caching it per process
     if (KktSmem<W, BW>::BYTES > 48 * 1024) {
-        const cudaError_t e = cudaFuncSetAttribute(kkt_band_kernel<W, BW, MINB, VIRT, DIAG, FUSE>, cudaFuncAttributeMaxDynamicSharedMemorySize, KktSmem<W, BW>::BYTES);
+        const cudaError_t e = cudaFuncSetAttribute(kkt_band_kernel<W, BW, VIRT, DIAG, FUSE>, cudaFuncAttributeMaxDynamicSharedMemorySize, KktSmem<W, BW>::BYTES);
         if (e != cudaSuccess) return e;
     }
-    kkt_band_kernel<W, BW, MINB, VIRT, DIAG, FUSE><<<(unsigned)((a->B + per_block - 1) / per_block), 128, KktSmem<W, BW>::BYTES, st>>>(*a);
+    kkt_band_kernel<W, BW, VIRT, DIAG, FUSE><<<(unsigned)((a->B + per_block - 1) / per_block), 128, KktSmem<W, BW>::BYTES, st>>>(*a);
     return cudaGetLastError();
 }
-template <int W, int BW, int MINB = (W == 16 ? 4 : 2)>
+template <int W, int BW>
 static cudaError_t launch_band_t(const dto_kkt_args* a, cudaStream_t st)
 {
-    constexpr int DEF = (W == 16 ? 4 : 2);
-    // candidate slots, the barrier diagonal and the fused right-hand side exist for the default occupancy only
-    if (a->diag) return a->virt ? launch_band_v<W, BW, DEF, true, true>(a, st) : launch_band_v<W, BW, DEF, false, true>(a, st);
-    if (a->virt) return launch_band_v<W, BW, DEF, true, false>(a, st);
-    if (a->fuse_rhs) return launch_band_v<W, BW, DEF, false, false, true>(a, st);
-    return launch_band_v<W, BW, MINB, false, false>(a, st);
+    if (a->diag) return a->virt ? launch_band_v<W, BW, true, true>(a, st) : launch_band_v<W, BW, false, true>(a, st);
+    if (a->virt) return launch_band_v<W, BW, true, false>(a, st);
+    if (a->fuse_rhs) return launch_band_v<W, BW, false, false, true>(a, st);
+    return launch_band_v<W, BW, false, false>(a, st);
 }
 template <int W, int BW, int M>
 static cudaError_t launch_band_s(const dto_kkt_args* a, cudaStream_t st)
@@ -699,12 +683,6 @@ extern "C" int dto_kkt_launch_band(const dto_kkt_args* a, void* stream)
     cudaError_t e = cudaErrorInvalidValue;
     const int bound = dto_kkt_bw_bound(a->W, a->bw);
     const bool two = a->variant != 2 || a->virt || a->diag;   // candidate slots / barrier diagonal: default kernel only
-    // experiment (DTO_KKT_VARIANT=occ5): 5 CTAs per SM, 96 registers, a few spills -- measured slower on every
-    // shape (cartpole 0.485 vs 0.346 ms, car 3.09 vs 2.35 ms; profiles/kkt_r01_history.jsonl tags v8 / v8occ5)
-    if (a->variant == 3 && !a->virt && !a->diag && a->W == 16 && (bound == 9 || bound == 15)) {
-        e = bound == 9 ? launch_band_t<16, 9, 5>(a, st) : launch_band_t<16, 15, 5>(a, st);
-        return e == cudaSuccess ? 1 : -(int)e;
-    }
     if (a->W == 16) {
         if (bound == 6) e = two ? launch_band_t<16, 6>(a, st) : launch_band_s<16, 6, 8>(a, st);
         else if (bound == 9) e = two ? launch_band_t<16, 9>(a, st) : launch_band_s<16, 9, 4>(a, st);

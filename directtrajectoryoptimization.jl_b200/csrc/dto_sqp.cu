@@ -163,7 +163,7 @@ __global__ void k_after_first(const dto_sqp_args a)
         if (done) atomicAdd(a.counters + DTO_SQP_N_DONE, 1);
         if (!done) a.alist[atomicAdd(a.counters + DTO_SQP_N_ACTIVE, 1)] = (int32_t)b;   // the next first factorisation skips the others
         if (bad) {
-            a.pred_next[atomicAdd(a.counters + DTO_SQP_N_BAD, 1)] = (int32_t)b;   // likely to need the correction again next time
+            atomicAdd(a.counters + DTO_SQP_N_BAD, 1);
             if (a.p.max_refactor > 0) atomicAdd(a.counters + DTO_SQP_N_RETRY, 1);
         }
     }
@@ -454,28 +454,16 @@ __global__ void k_reg_ladder(const dto_sqp_args a, int32_t m)
     a.tries[b] += left < m ? left : m;
 }
 
-// prediction (before this iteration's first factorisation is known): the ladder a listed problem WOULD climb if its
-// damping lm turns out not to be enough -- delta = lm and first = true are what k_reg_ladder would see after the check
-__global__ void k_pred_ladder(const dto_sqp_args a, int32_t count, int32_t m)
-{
-    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= count) return;
-    const int64_t b = a.pred_cur[k];
-    ladder_values(a, b, a.delta[b], true, m, a.p.max_refactor, k, a.vreg2, a.vidx2);
-}
-
 // block per listed problem: the first candidate with N_c negative pivots and a finite solution is kept
-template <bool PRED>
 __global__ void __launch_bounds__(256) k_pick(const dto_sqp_args a, int32_t count, int32_t m)
 {
     __shared__ int s_pick, s_good;
     const int64_t k = blockIdx.x;
-    const int64_t b = PRED ? a.pred_cur[k] : a.idx[k];
-    if (PRED && !a.bad[b]) return;        // the damping was enough after all: the candidates are dropped
-    const double* __restrict__ vreg = PRED ? a.vreg2 : a.vreg;
-    const double* __restrict__ vsol = PRED ? a.vsol2 : a.vsol;
-    const int32_t* __restrict__ vnneg = PRED ? a.vnneg2 : a.vnneg;
-    const double* __restrict__ vL = PRED ? a.vL2 : a.vL;
+    const int64_t b = a.idx[k];
+    const double* __restrict__ vreg = a.vreg;
+    const double* __restrict__ vsol = a.vsol;
+    const int32_t* __restrict__ vnneg = a.vnneg;
+    const double* __restrict__ vL = a.vL;
     if (threadIdx.x < 32) {
         const int lane = threadIdx.x;
         int pick = m - 1, good = 0;
@@ -496,15 +484,8 @@ __global__ void __launch_bounds__(256) k_pick(const dto_sqp_args a, int32_t coun
             a.preg[b] = vreg[v];
             a.nneg_w[b] = vnneg[v];
             a.bad[b] = good ? 0 : 1;
-            if (PRED) {
-                a.first[b] = 0;
-                a.tries[b] = m < a.p.max_refactor ? m : a.p.max_refactor;
-                // k_after_first counted this problem as bad with tries left: no longer, if repaired or out of tries
-                if (good || a.tries[b] >= a.p.max_refactor) atomicSub(a.counters + DTO_SQP_N_RETRY, 1);
-            } else {
-                if (!good) atomicAdd(a.counters + DTO_SQP_N_BAD, 1);
-                if (!good && a.tries[b] < a.p.max_refactor) atomicAdd(a.counters + DTO_SQP_N_RETRY, 1);
-            }
+            if (!good) atomicAdd(a.counters + DTO_SQP_N_BAD, 1);
+            if (!good && a.tries[b] < a.p.max_refactor) atomicAdd(a.counters + DTO_SQP_N_RETRY, 1);
         }
     }
     __syncthreads();
@@ -646,7 +627,7 @@ __global__ void k_ip_after_first(const dto_sqp_args a)
         if (done) atomicAdd(a.counters + DTO_SQP_N_DONE, 1);
         if (!done) a.alist[atomicAdd(a.counters + DTO_SQP_N_ACTIVE, 1)] = (int32_t)b;
         if (bad) {
-            a.pred_next[atomicAdd(a.counters + DTO_SQP_N_BAD, 1)] = (int32_t)b;
+            atomicAdd(a.counters + DTO_SQP_N_BAD, 1);
             if (a.p.max_refactor > 0) atomicAdd(a.counters + DTO_SQP_N_RETRY, 1);
         }
     }
@@ -970,21 +951,7 @@ extern "C" int dto_sqp_k_reg_ladder(const dto_sqp_args* a, int32_t m, void* s)
 extern "C" int dto_sqp_k_reg_pick(const dto_sqp_args* a, int32_t count, int32_t m, void* s)
 {
     if (count <= 0) return 0;
-    k_pick<false><<<(unsigned)count, 256, 0, (cudaStream_t)s>>>(*a, count, m);
-    const cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : -(int)e;
-}
-extern "C" int dto_sqp_k_pred_ladder(const dto_sqp_args* a, int32_t count, int32_t m, void* s)
-{
-    if (count <= 0) return 0;
-    k_pred_ladder<<<(unsigned)((count + 127) / 128), 128, 0, (cudaStream_t)s>>>(*a, count, m);
-    const cudaError_t e = cudaGetLastError();
-    return e == cudaSuccess ? 0 : -(int)e;
-}
-extern "C" int dto_sqp_k_pred_pick(const dto_sqp_args* a, int32_t count, int32_t m, void* s)
-{
-    if (count <= 0) return 0;
-    k_pick<true><<<(unsigned)count, 256, 0, (cudaStream_t)s>>>(*a, count, m);
+    k_pick<<<(unsigned)count, 256, 0, (cudaStream_t)s>>>(*a, count, m);
     const cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? 0 : -(int)e;
 }

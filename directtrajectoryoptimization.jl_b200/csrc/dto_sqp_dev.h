@@ -67,15 +67,6 @@ typedef struct dto_sqp_args {
     int64_t factor_stride;
     int32_t* tries;       /* [B] inertia-correction tries used by the problem in this iteration */
     int32_t* alist;       /* [B] problems that have not converged (written by the first check, for the next iteration) */
-    /* prediction: the problems whose first factorisation had the wrong inertia in the previous iteration get their ladder
-     * factorised in a second set of candidate slots WHILE the first factorisation of this iteration runs */
-    int32_t* pred_cur;    /* [B] list used in this iteration                                   */
-    int32_t* pred_next;   /* [B] list written by this iteration's first check                  */
-    int32_t* vidx2;       /* second candidate set, as above                                    */
-    double* vreg2;
-    double* vsol2;
-    int32_t* vnneg2;
-    double* vL2;
     /* interior-point mode */
     const double *hasL, *hasU, *lo, *up;   /* [N_z] 0/1 masks and finite bound values (0 where absent)        */
     const double* hasI;                    /* [N_c] 1 = inequality row c_i(z) <= 0                              */
@@ -117,10 +108,6 @@ int dto_sqp_k_ip_after_first(const dto_sqp_args* a, void* stream);
 int dto_sqp_k_ip_direction(const dto_sqp_args* a, void* stream);
 int dto_sqp_k_ip_ls_round(const dto_sqp_args* a, int32_t round, void* stream);
 int dto_sqp_k_ip_end(const dto_sqp_args* a, void* stream);
-/* prediction: ladder of the first `count` problems of pred_cur from their damping (before the first factorisation is known) */
-int dto_sqp_k_pred_ladder(const dto_sqp_args* a, int32_t count, int32_t m, void* stream);
-/* after the first check: a predicted problem that did turn out bad takes the first working candidate of the second set */
-int dto_sqp_k_pred_pick(const dto_sqp_args* a, int32_t count, int32_t m, void* stream);
 /* knot-block damped BFGS: update every block from s = z - zp, y = (g + J'lam) - (gp + Jp'lam), then zp, gp, Jp = z, g, J */
 int dto_sqp_k_qn_update(const dto_sqp_args* a, void* stream);
 /* slot k * R + j (k-th entry of oidx, j < R) <- z + alpha 2^-j dz and the problem's parameters */

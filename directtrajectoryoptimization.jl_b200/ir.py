@@ -740,9 +740,10 @@ def _needs_pool(v: float) -> bool:
 
 def emit(g: Graph, outputs: List[Tuple[str, int]], load: Dict[Tuple[str, int], str], indent: str = "    ",
          prefix: str = "t", cpool: Optional[Dict[float, int]] = None, cname: str = "dto_k", order: int = 0,
-         bf: bool = False, live_cap: int = 56) -> List[str]:
+         bf: bool = False) -> List[str]:
     """Straight-line C for the nodes reachable from `outputs` [(lhs, node)], DFS post-order in
-    output order (keeps live ranges short); sin/cos of one argument become one sincos().
+    output order (keeps live ranges short), or with order=2 register-pressure-aware list scheduling; sin/cos of one
+    argument become one sincos().
     bf=True: sin/cos/reciprocal use the branch-free device functions dto_sincos_bf / dto_rcp_bf, which
     OR a flag into the local `dto_bad` when an argument is outside their domain (the caller then
     re-evaluates with the library functions): the whole program becomes ONE basic block, so ptxas can
@@ -830,7 +831,7 @@ def emit(g: Graph, outputs: List[Tuple[str, int]], load: Dict[Tuple[str, int], s
             name[n] = nm
             lines.append(f"{indent}const double {nm} = {op}({ref(a[0])});")
 
-    if order in (2, 3):
+    if order == 2:
         # register-pressure-aware list scheduling: among the ready nodes pick the one that retires the
         # most live values (last uses) -- ptxas largely keeps source order for long FP64 blocks, so
         # the emitted order decides how many registers the ~1000-instruction knot program needs
@@ -871,31 +872,16 @@ def emit(g: Graph, outputs: List[Tuple[str, int]], load: Dict[Tuple[str, int], s
                     stored.add(lhs)
 
         flush_outputs()
-        # order 3: critical-path-first list scheduling under a cap on live values -- two in-order warps per
-        # sub-partition cannot hide the FP64 latency by themselves, so independent chains are interleaved in the
-        # SOURCE order (ptxas keeps long FP64 blocks largely in order); above the cap the pressure rule takes over
-        height: Dict[int, int] = {}
-        if order == 3:
-            lat = {"rcp": 6, "sin": 12, "cos": 12, "powi": 2}
-            for n in reversed(nodes):
-                height[n] = lat.get(g.op[n], 1) + max([height[c_] for c_ in consumers[n]], default=0)
-        live = 0
         while ready:
             best, best_key = None, None
-            over = order == 3 and live >= live_cap
             for n in ready:
                 frees = sum(1 for a in set(ops_of[n]) if uses[a] == 1)
                 creates = 0 if (not consumers[n]) else 1
-                if order == 3 and not over:
-                    # longest remaining path first; among equals the one that frees most, not the chain just extended
-                    key = (height[n], frees - creates, 0 if last_pick in ops_of[n] else 1, -order_idx[n])
-                else:
-                    # prefer: most net frees, then consumers of the value defined last (chains), then source order
-                    key = (frees - creates, 1 if last_pick in ops_of[n] else 0, -order_idx[n])
+                # prefer: most net frees, then consumers of the value defined last (chains), then source order
+                key = (frees - creates, 1 if last_pick in ops_of[n] else 0, -order_idx[n])
                 if best_key is None or key > best_key:
                     best, best_key = n, key
             n = best
-            live += (1 if consumers[n] else 0) - sum(1 for a in set(ops_of[n]) if uses[a] == 1)
             ready.remove(n)
             define(n)
             if g.op[n] in ("sin", "cos") and g.args[n][0] in paired:  # sincos defines both
@@ -921,20 +907,6 @@ def emit(g: Graph, outputs: List[Tuple[str, int]], load: Dict[Tuple[str, int], s
             flush_outputs()
         flush_outputs()
         assert len(stored) == len(outputs), "scheduler left outputs unstored"
-        return lines
-    if order == 1:
-        # level order: every node at its dependency depth (maximal ILP in source order; ptxas then
-        # trades it against registers), outputs stored as soon as their node exists
-        depth: Dict[int, int] = {}
-        for n in sorted(need):
-            depth[n] = 1 + max([depth[a] for a in g.args[n]], default=0) if g.op[n] not in ("const",) else 0
-        pending: Dict[int, List[str]] = {}
-        for lhs, root in outputs:
-            pending.setdefault(root, []).append(lhs)
-        for n in sorted((n for n in need if g.op[n] not in ("const", "neg")), key=lambda n: (depth[n], n)):
-            define(n)
-        for lhs, root in outputs:
-            lines.append(f"{indent}{lhs} = {ref(root)};")
         return lines
     # iterative DFS post-order
     for lhs, root in outputs:

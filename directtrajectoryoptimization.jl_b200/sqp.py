@@ -863,7 +863,7 @@ def solve_native(nlp, z0, lam0=None, options: Optional[SQPOptions] = None) -> SQ
     res = SQPResult(z, lam, iters.astype(np.float64), done.astype(bool), cv, dr, f, [])
     res.staged = done == 2          # converged by the bound continuation (see solve_bounded)
     res.stats = dict(iterations=int(stats[0]), launches=int(stats[1]), factorisations=int(stats[2]), syncs=int(stats[3]),
-                     refactorisations=int(stats[4]), corrections=int(stats[5]), search_rounds=int(stats[6]), multi_trial_passes=int(stats[7]), predicted_passes=int(stats[15]),
+                     refactorisations=int(stats[4]), corrections=int(stats[5]), search_rounds=int(stats[6]), multi_trial_passes=int(stats[7]),
                      phase_ms=dict(callbacks_first_factor=stats[8] / 1e3, inertia_correction=stats[9] / 1e3, line_search=stats[10] / 1e3,
                                    of_which_corrections=stats[11] / 1e3, setup=stats[12] / 1e3, loop=stats[13] / 1e3,
                                    results=stats[14] / 1e3))

@@ -309,7 +309,7 @@ void dto_sqp_default_options(dto_sqp_options* o);
  * one-pass evaluations of all remaining step lengths, and host
  * microseconds spent in: callbacks + first factorisation, inertia correction, line search (with corrections),
  * second-order corrections; set-up (allocations, tables, host -> device), iteration loop, results (device -> host);
- * iterations whose predicted inertia corrections ran beside the first factorisation} -- summed over the direct solve and the
+ * reserved, always 0} -- summed over the direct solve and the
  * two passes of the bound continuation when that ran. The final iterate stays resident as the batch's z (dto_get_last_x). */
 int dto_sqp_solve(dto_batch* b, const dto_sqp_options* options, const double* z0, const double* lambda0, const double* lower,
                   const double* upper, double* z, double* lambda, int32_t* iterations, uint8_t* converged,

@@ -13,7 +13,7 @@ from examples import models as M
 from golden.make_golden import GOLDEN, tag
 from oracle import api as O
 from oracle import cgen
-from util import assert_close, make_inputs
+from util import KERNEL_VARIANTS, assert_close, make_inputs
 
 pytestmark = pytest.mark.gpu
 HERE = os.path.join(os.path.dirname(__file__), "golden")
@@ -241,8 +241,6 @@ def test_table_gather_fallback_matches(monkeypatch):
     assert pn.compiled_gather()
 
 
-KERNEL_VARIANTS = ["ws=0,persist=0", "ws=0,ws_min_ops=0", "ws_min_ops=0,ws_all=1", "ws_min_ops=0,ws_plan=0", "ws_min_ops=0,bf=0,emit=0",
-                   "ws_min_ops=0,ws_helpers=4"]
 VARIANT_MODELS = [("pendulum", dict(), 1), ("cartpole", dict(T=11), 2), ("acrobot", dict(T=9), 3),
                   ("car", dict(T=12, obstacle="general"), 4)]
 
@@ -300,7 +298,7 @@ def test_branch_free_math_falls_back_outside_its_domain(monkeypatch):
     z[4, 11] = np.inf
     z[5, 1] = 2.0 ** 31    # boundary of the fast path
     res = {}
-    for t in ("ws_min_ops=0,bf=0,emit=0", ""):
+    for t in ("bf=0,emit=0", ""):
         if t:
             monkeypatch.setenv("DTO_TUNE", t)
         else:
@@ -310,7 +308,7 @@ def test_branch_free_math_falls_back_outside_its_domain(monkeypatch):
         pn.close()
     monkeypatch.delenv("DTO_TUNE", raising=False)
     for k in ("c", "J", "H"):
-        a, b = res[""][k], res["ws_min_ops=0,bf=0,emit=0"][k]
+        a, b = res[""][k], res["bf=0,emit=0"][k]
         assert np.array_equal(np.isnan(a), np.isnan(b)), f"{k}: NaN pattern differs"
         fin = np.isfinite(b)
         assert_close(f"bf=1 {k}", a[fin], b[fin], rtol=1e-12, atol=1e-14)

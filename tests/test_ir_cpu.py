@@ -113,3 +113,15 @@ def test_user_jacobian_is_what_gets_lowered(mode, monkeypatch):
         inp = {("y", 0): 0.1, ("y", 1): 0.2, ("x", 0): 0.7, ("x", 1): -0.4, ("u", 0): 0.3}
         vals = g.evaluate(nodes, inp)
         assert abs(vals[1] - 3.0 * 0.1 * np.cos(0.7)) < 1e-15 and len(vals) == 10
+
+
+@pytest.mark.parametrize("tune", ["pdl_plain=0", "emit=1", "ws_helpers=3", "ws=yes", "ws"])
+def test_unsupported_tuning_is_refused(tune, monkeypatch):
+    """A retired or misspelt DTO_TUNE key, or a value no build supports, is an error naming the accepted keys: it must
+    not build the default kernels under a new content hash."""
+    monkeypatch.setenv("DTO_TUNE", tune)
+    with pytest.raises(ValueError, match=r"accepted: ws=1\|0, persist=1\|0"):
+        codegen._tuning()
+    monkeypatch.setenv("DTO_TUNE", "ws=0, persist=0")
+    t = codegen._tuning()
+    assert (t["ws"], t["persist"], t["emit"]) == (0, 0, 2)

@@ -10,6 +10,10 @@ from oracle import api as O
 
 RTOL, ATOL = 1e-12, 1e-14   # BASELINE.json north_star: 1e-12 relative or 1e-14 absolute
 
+# DTO_TUNE kernel-selection variants the GPU tests compare against the default build (test_gpu_properties.py); build()
+# compiles their model libraries ahead of the tests
+KERNEL_VARIANTS = ["ws=0,persist=0", "ws=0", "ws_all=1", "ws_plan=0", "bf=0,emit=0", "ws_helpers=4"]
+
 
 def rng_for(config: int, shard: int = 0):
     return np.random.default_rng(20261017 + 1000 * config + shard)

@@ -57,7 +57,7 @@ def run_native(model, nlp, z0, o, name, B, T, max_iter):
             "objective": {"median": float(np.median(f)), "min": float(f.min()), "max": float(f.max())},
             "cv_max_accepted": float(cv[ok].max()) if ok.any() else None, "dual_residual_median": float(np.median(res.dual_residual)),
             "gpu_launches": res.stats["launches"], "factorisations": res.stats["factorisations"], "host_syncs": res.stats["syncs"],
-            "refactorisations": res.stats["refactorisations"], "corrections": res.stats["corrections"], "search_rounds": res.stats["search_rounds"], "multi_trial_passes": res.stats["multi_trial_passes"], "predicted_passes": res.stats["predicted_passes"], "phase_ms": res.stats["phase_ms"],
+            "refactorisations": res.stats["refactorisations"], "corrections": res.stats["corrections"], "search_rounds": res.stats["search_rounds"], "multi_trial_passes": res.stats["multi_trial_passes"], "phase_ms": res.stats["phase_ms"],
             "iterations_run": res.stats["iterations"], "ms_per_iteration": 1e3 * dt / max(1, res.stats["iterations"])}
 
 

@@ -7,8 +7,7 @@ import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-TUNES = ["warps=4,min_ctas=1", "warps=4,min_ctas=2", "warps=4,min_ctas=3", "warps=4,min_ctas=4", "warps=2,min_ctas=8",
-         "warps=8,min_ctas=2", "warps=2,min_ctas=6", "warps=1,min_ctas=12"]
+TUNES = ["", "ws=0,persist=0", "ws=0", "ws_all=1", "ws_plan=0", "bf=0,emit=0", "ws_helpers=4"]   # codegen.TUNE_VALUES
 
 CHILD = r"""
 import sys, os, json, time
