@@ -78,27 +78,8 @@ __device__ __forceinline__ double row_shift(const dto_kkt_args& a, size_t row, i
     return reg;
 }
 
-// right-hand-side entry of original row ip (natural order): read from the rhs array written by kkt_rhs_kernel, or
-// (a.fuse_rhs) computed here with the same operations in the same order -- the reference's loop
-// (examples/pendulum/pendulum.jl:155-173): cy = sum over constraint rows ascending of C[j,i]*y[j]; h[i] = grad[i] + cy
-__device__ __forceinline__ double rhs_entry(const dto_kkt_args& a, int64_t b, int32_t ip, const double* __restrict__ hb, bool valid)
-{
-    if (ip < 0) return 0.0;
-    if (!a.fuse_rhs) return hb[ip];
-    double h;
-    if (ip < a.N_z) {
-        const double* __restrict__ Jb = a.J + b * a.nnz_J;
-        const double* __restrict__ yb = a.y + b * a.N_c;
-        double cy = 0.0;
-        for (int k = a.colptr[ip]; k < a.colptr[ip + 1]; ++k) cy = __dadd_rn(cy, __dmul_rn(Jb[a.colslot[k]], yb[a.colrow[k]]));
-        h = __dadd_rn(a.g[b * a.N_z + ip], cy);
-        if (a.fixed != nullptr && a.fixed[ip]) h = 0.0;
-    } else {
-        h = a.c[b * a.N_c + (ip - a.N_z)];
-    }
-    if (valid) a.rhs[b * a.dim + ip] = h;
-    return h;
-}
+// right-hand-side entry of original row ip (natural order, from kkt_rhs_kernel's array hb); padding rows (ip < 0) read 0
+__device__ __forceinline__ double rhs_entry(const double* __restrict__ hb, int32_t ip) { return ip < 0 ? 0.0 : hb[ip]; }
 
 template <int W, bool DIAG = false>
 __device__ __forceinline__ void load_rows(const dto_kkt_args& a, const double* __restrict__ Hb, const double* __restrict__ JbmH,
@@ -131,7 +112,7 @@ struct KktSmem {
     static constexpr int BYTES = 4 * NG * PER_GROUP;        // 4 warps per CTA
 };
 
-// ---------------- backward solve: x = L^-T y (shared by both factor kernels) ----------------
+// ---------------- backward solve: x = L^-T y (shared by the factor and resolve kernels) ----------------
 template <int W, int BW>
 __device__ __forceinline__ void kkt_backward(const dto_kkt_args& a, unsigned char* gsm, const double* Lg, const double* Yg, int nblk, int i,
                                              bool valid, int64_t b)
@@ -216,9 +197,7 @@ __device__ __forceinline__ void kkt_backward(const dto_kkt_args& a, unsigned cha
 // VIRT = candidate launch (dto_kkt_args::virt): outputs and regularisation indexed by slot. A separate instantiation: as a
 // run-time switch its extra live index cost the default path registers and spills (acrobot, 64 problems: 0.275 vs 0.204 ms)
 // DIAG = a per-problem, per-variable diagonal is added to the Hessian block (dto_kkt_args::diag); separate for the same reason
-// FUSE = the kernel computes the right-hand side itself (dto_kkt_args::fuse_rhs, an option measured slower): its own instantiation too --
-// carrying the code path costs the default kernel 4 % on cartpole (registers)
-template <int W, int BW, bool VIRT = false, bool DIAG = false, bool FUSE = false>
+template <int W, int BW, bool VIRT = false, bool DIAG = false>
 __global__ void __launch_bounds__(128, (W == 16 ? 4 : 2)) kkt_band_kernel(const dto_kkt_args a)
 {
     constexpr int G = W;
@@ -243,20 +222,14 @@ __global__ void __launch_bounds__(128, (W == 16 ? 4 : 2)) kkt_band_kernel(const 
     double* stage = reinterpret_cast<double*>(gsm);                              // forward: rows of block blk+2, [w][i]
     double (*lcol)[W] = reinterpret_cast<double (*)[W]>(gsm + SM::RING * SM::SLOT);  // un-scaled column, double-buffered
 
-    // right-hand-side entry of original row ip; a candidate launch always finds it in the rhs array (nothing it depends
-    // on changed since the launch that wrote it), which also keeps the problem index out of the loop's live registers
-    auto rhs_at = [&](int32_t ip) -> double {
-        if (VIRT || !FUSE) return ip < 0 ? 0.0 : hb[ip];
-        return rhs_entry(a, b, ip, hb, valid);
-    };
     double A[W], Bv[W];
     double ra, rb = 0.0, rc = 0.0, regc = 0.0;
     int32_t nidx[W];                                  // gather indices of the rows two blocks ahead
     load_rows<W, DIAG>(a, Hb, Jb, 0, i, A, bo, b);
-    ra = rhs_at(a.iperm[i]);
+    ra = rhs_entry(hb, a.iperm[i]);
     if (nblk > 1) {
         load_rows<W, DIAG>(a, Hb, Jb, 1, i, Bv, bo, b);
-        rb = rhs_at(a.iperm[W + i]);
+        rb = rhs_entry(hb, a.iperm[W + i]);
     } else {
 #pragma unroll
         for (int w = 0; w < W; ++w) Bv[w] = 0.0;
@@ -301,12 +274,7 @@ __global__ void __launch_bounds__(128, (W == 16 ? 4 : 2)) kkt_band_kernel(const 
                 cp_async8_zfill(stage + w * W + i, sx >= 0 ? (const void*)(bp + sx) : (const void*)Hb, sx >= 0 ? 8 : 0);
             }
             cp_async_commit();
-            if (FUSE) {
-                rc = rhs_at(ipn);
-            } else {
-                rc = 0.0;
-                if (ipn >= 0) rc = hb[ipn];
-            }
+            rc = rhs_entry(hb, ipn);
             regc = (fixn || ipn < 0) ? 1.0 : (ipn < a.N_z ? prim : -a.dual_reg);   // = row_shift(): the values of the dreg table
             if (DIAG && !fixn && ipn >= 0) regc += a.diag[b * a.dim + ipn];
             load_idx(blk + 3);
@@ -375,144 +343,6 @@ __global__ void __launch_bounds__(128, (W == 16 ? 4 : 2)) kkt_band_kernel(const 
 }
 
 // ------------------------------------------------------------------------------------------------
-// Single-row-set factor kernel (half bandwidth BW <= W - M, M in {4, 8}).
-// A lane's row of block blk is finished right after step s = i, and its row of block blk+1 is first
-// touched at step i + (W - BW) >= i + M, so ONE register row per lane is enough if lanes hand over to
-// their next row in batches of M: at step t = M, 2M, .., W the lanes [t - M, t) store their finished
-// y value and take their next row from the shared-memory stage that cp.async filled one block earlier.
-// Per elimination step every lane then has at most one live row: one select, one multiply by 1/d, one
-// shared-memory store of the un-scaled column entry (slot (i - s - 1) mod W; the pivot lane uses the
-// free slot W - 1 to broadcast its right-hand-side entry), one predicated store of the L entry, and BW
-// DFMAs -- about half the instructions of the two-set kernel above.
-template <int W, int BW>
-struct KktSmemS {
-    using B = KktSmem<W, BW>;
-    static constexpr int AREA = (B::RING * B::SLOT > 2 * W * W * 8) ? B::RING * B::SLOT : 2 * W * W * 8;
-    static constexpr int PER_GROUP = AREA + 2 * W * 8;
-    static constexpr int BYTES = 4 * B::NG * PER_GROUP;
-};
-
-template <int W, int BW, int M>
-__global__ void __launch_bounds__(128, (W == 16 ? 4 : 2)) kkt_band_kernel_s(const dto_kkt_args a)
-{
-    static_assert(M <= W - BW && W % M == 0 && BW <= W - 3, "hand-over period must not exceed W - BW; slot W-1 must be free");
-    constexpr int G = W;
-    using SM = KktSmem<W, BW>;
-    using SS = KktSmemS<W, BW>;
-    constexpr int LW = SM::LW;
-    extern __shared__ __align__(16) unsigned char kkt_smem[];
-    const int lane = threadIdx.x & 31;
-    const int wib = threadIdx.x >> 5;
-    const int grp = lane / G, i = lane % G;
-    const int64_t b0 = ((int64_t)blockIdx.x * 4 + wib) * SM::NG + grp;
-    const bool valid = b0 < a.B;
-    const int64_t bs = valid ? b0 : a.B - 1;
-    const int64_t b = a.pidx ? (int64_t)a.pidx[bs] : bs;
-    const double* Hb = a.H + b * a.nnz_H;
-    const double* Jb = a.J + b * a.nnz_J - a.nnz_H;  // see load_rows
-    const double* hb = a.rhs + b * a.dim;
-    const int nblk = a.nblk;
-    double* Lg = a.L + (size_t)b * a.factor_stride;
-    double* Yg = Lg + (size_t)nblk * W * LW;
-    unsigned char* gsm = kkt_smem + (size_t)(wib * SM::NG + grp) * SS::PER_GROUP;
-    double* stage = reinterpret_cast<double*>(gsm);                        // [2][W][W]: rows of blocks blk+1 / blk+2
-    double (*lcol)[W] = reinterpret_cast<double (*)[W]>(gsm + SS::AREA);   // un-scaled column, double-buffered
-
-    double R[W];
-    double rr;
-    double rn1 = 0.0, regn1 = 1.0, rn2 = 0.0, regn2 = 1.0;   // rhs / diagonal shift of this lane's rows in blocks blk+1, blk+2
-    int32_t nidx[W];
-    load_rows<W>(a, Hb, Jb, 0, i, R, b);
-    rr = rhs_entry(a, b, a.iperm[i], hb, valid);
-    auto load_idx = [&](int blk) {
-        if (blk < nblk) {
-            const int32_t* src = a.src + ((size_t)blk * W) * W + i;
-#pragma unroll
-            for (int w = 0; w < W; ++w) nidx[w] = src[w * W];
-        }
-    };
-    // gather the rows of block `blk` (indices in nidx) into stage[blk & 1]; always commits one group
-    auto issue_rows = [&](int blk, double& rn, double& regn) {
-        if (blk < nblk) {
-            double* st = stage + (blk & 1) * W * W;
-#pragma unroll
-            for (int w = 0; w < W; ++w) {
-                const int32_t sx = nidx[w];
-                const double* bp = (sx < a.nnz_H) ? Hb : Jb;
-                cp_async8_zfill(st + w * W + i, sx >= 0 ? (const void*)(bp + sx) : (const void*)Hb, sx >= 0 ? 8 : 0);
-            }
-            rn = rhs_entry(a, b, a.iperm[(size_t)blk * W + i], hb, valid);
-            regn = row_shift(a, (size_t)blk * W + i, b);
-        }
-        cp_async_commit();
-    };
-    load_idx(1);
-    issue_rows(1, rn1, regn1);
-    load_idx(2);
-
-    for (int blk = 0; blk < nblk; ++blk) {
-        issue_rows(blk + 2, rn2, regn2);          // consumed during block blk + 1
-        load_idx(blk + 3);
-        const bool has_next = blk + 1 < nblk;
-        double* stn = stage + ((blk + 1) & 1) * W * W + i;
-        double* LA = Lg + (size_t)blk * W * LW;
-        bool staged = false;
-#pragma unroll
-        for (int s = 0; s < G; ++s) {
-            const int p = s & (W - 1);
-            // lanes below the last hand-over point already hold their row of block blk+1
-            const bool live = (i > s) || (i < (s & ~(M - 1)));
-            const double v = live ? R[p] : 0.0;
-            double* vs = lcol[s & 1];
-            vs[(i - s - 1) & (W - 1)] = v;                       // lane s (v = 0) lands on the free slot W-1 ...
-            if (i == s) vs[W - 1] = rr;                          // ... which carries y_j instead
-            const double d = shfl_g<G>(R[p], s);
-            const double dinv = 1.0 / d;
-            const double l = v * dinv;
-            const int qi = (i - s) & (W - 1);                   // row - j
-            if (valid && qi >= 1 && qi <= BW) LA[s * LW + qi] = l;
-            if (valid && i == s) LA[s * LW] = d;
-            __syncwarp();
-            const double yj = vs[W - 1];
-            rr = fma(-l, yj, rr);
-            if (i == s) rr = yj * dinv;
-            const double nl = -l;
-#pragma unroll
-            for (int q = 1; q <= BW; ++q) R[(p + q) & (W - 1)] = fma(nl, vs[q - 1], R[(p + q) & (W - 1)]);
-            if (((s + 1) & (M - 1)) == 0) {
-                // hand-over: lanes [s + 1 - M, s] have finished their row of this block
-                if (!staged) {
-                    cp_async_wait<1>();                          // this lane's copies of block blk+1 have landed
-                    __syncwarp();
-                    // reference: K[i,i] += primal_reg / -= dual_reg after the assignment; each lane fixes the
-                    // diagonal entry of ITS row in the stage (slot w = i), or clears its row past the last block
-                    if (has_next) {
-                        stn[i * W] += regn1;
-                    } else {
-#pragma unroll
-                        for (int w = 0; w < W; ++w) stage[((blk + 1) & 1) * W * W + w * W + i] = 0.0;
-                    }
-                    staged = true;
-                }
-                if (i >= s + 1 - M && i <= s) {
-                    if (valid) Yg[(size_t)blk * W + i] = rr;
-#pragma unroll
-                    for (int w = 0; w < W; ++w) R[w] = stn[w * W];
-                    rr = has_next ? rn1 : 0.0;
-                }
-            }
-        }
-        rn1 = rn2;
-        regn1 = regn2;
-        __syncwarp();   // every lane has taken its row: stage[(blk+1)&1] may be refilled (block blk+3) next iteration
-    }
-    cp_async_wait<0>();
-    __syncwarp();
-    __threadfence_block();
-    kkt_backward<W, BW>(a, gsm, Lg, Yg, nblk, i, valid, b);
-}
-
-// ------------------------------------------------------------------------------------------------
 // Solve again with the factor of the last factorisation: K unchanged, new right-hand side (a second-order
 // correction re-solves with c(z) + c(z + dz), Nocedal & Wright 18.3). The forward substitution reads the stored
 // columns of L block by block through the same 3-slot cp.async ring the backward solve uses and applies the
@@ -550,17 +380,11 @@ __global__ void __launch_bounds__(128, (W == 16 ? 4 : 2)) kkt_resolve_kernel(con
     issue(0);
     issue(1);
     issue(2);
-    double ra = rhs_entry(a, b, a.iperm[i], hb, valid);
-    double rb = nblk > 1 ? rhs_entry(a, b, a.iperm[W + i], hb, valid) : 0.0;
+    double ra = rhs_entry(hb, a.iperm[i]);
+    double rb = nblk > 1 ? rhs_entry(hb, a.iperm[W + i]) : 0.0;
     int32_t ipn = nblk > 2 ? a.iperm[2 * W + i] : -1;   // source row of the block two ahead, fetched one block early
     for (int blk = 0; blk < nblk; ++blk) {
-        double rc = 0.0;
-        if (blk + 2 < nblk) {
-            if (a.fuse_rhs)
-                rc = rhs_entry(a, b, ipn, hb, valid);
-            else if (ipn >= 0)
-                rc = hb[ipn];
-        }
+        const double rc = blk + 2 < nblk ? rhs_entry(hb, ipn) : 0.0;
         if (blk + 3 < nblk) ipn = a.iperm[(size_t)(blk + 3) * W + i];
         cp_async_wait<2>();
         __syncwarp();
@@ -641,86 +465,63 @@ extern "C" int dto_kkt_launch_rhs(const dto_kkt_args* a, void* stream)
     return e == cudaSuccess ? 1 : -(int)e;
 }
 
-template <int W, int BW, bool VIRT, bool DIAG, bool FUSE = false>
-static cudaError_t launch_band_v(const dto_kkt_args* a, cudaStream_t st)
+using kkt_kernel_t = void (*)(dto_kkt_args);
+
+// the factor kernel instantiation for the launch's options
+struct BandKernel {
+    template <int W, int BW>
+    static kkt_kernel_t get(const dto_kkt_args* a)
+    {
+        if (a->diag) return a->virt ? kkt_band_kernel<W, BW, true, true> : kkt_band_kernel<W, BW, false, true>;
+        return a->virt ? kkt_band_kernel<W, BW, true, false> : kkt_band_kernel<W, BW, false, false>;
+    }
+};
+struct ResolveKernel {
+    template <int W, int BW>
+    static kkt_kernel_t get(const dto_kkt_args*) { return kkt_resolve_kernel<W, BW>; }
+};
+
+// one CTA = 4 warps = 4 * 32 / W problems, with the KktSmem<W, BW> layout in dynamic shared memory
+template <class Kernel, int W, int BW>
+static cudaError_t launch_at(const dto_kkt_args* a, cudaStream_t st)
 {
+    const kkt_kernel_t kernel = Kernel::template get<W, BW>(a);
     const int64_t per_block = 4 * (32 / W);
     // the opt-in is per device and a batch may span several: set it on every launch (a cheap driver call
     // next to a >= 100 us kernel) instead of caching it per process
     if (KktSmem<W, BW>::BYTES > 48 * 1024) {
-        const cudaError_t e = cudaFuncSetAttribute(kkt_band_kernel<W, BW, VIRT, DIAG, FUSE>, cudaFuncAttributeMaxDynamicSharedMemorySize, KktSmem<W, BW>::BYTES);
+        const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, KktSmem<W, BW>::BYTES);
         if (e != cudaSuccess) return e;
     }
-    kkt_band_kernel<W, BW, VIRT, DIAG, FUSE><<<(unsigned)((a->B + per_block - 1) / per_block), 128, KktSmem<W, BW>::BYTES, st>>>(*a);
-    return cudaGetLastError();
-}
-template <int W, int BW>
-static cudaError_t launch_band_t(const dto_kkt_args* a, cudaStream_t st)
-{
-    if (a->diag) return a->virt ? launch_band_v<W, BW, true, true>(a, st) : launch_band_v<W, BW, false, true>(a, st);
-    if (a->virt) return launch_band_v<W, BW, true, false>(a, st);
-    if (a->fuse_rhs) return launch_band_v<W, BW, false, false, true>(a, st);
-    return launch_band_v<W, BW, false, false>(a, st);
-}
-template <int W, int BW, int M>
-static cudaError_t launch_band_s(const dto_kkt_args* a, cudaStream_t st)
-{
-    const int64_t per_block = 4 * (32 / W);
-    if (KktSmemS<W, BW>::BYTES > 48 * 1024) {
-        const cudaError_t e = cudaFuncSetAttribute(kkt_band_kernel_s<W, BW, M>, cudaFuncAttributeMaxDynamicSharedMemorySize, KktSmemS<W, BW>::BYTES);
-        if (e != cudaSuccess) return e;
-    }
-    kkt_band_kernel_s<W, BW, M><<<(unsigned)((a->B + per_block - 1) / per_block), 128, KktSmemS<W, BW>::BYTES, st>>>(*a);
+    kernel<<<(unsigned)((a->B + per_block - 1) / per_block), 128, KktSmem<W, BW>::BYTES, st>>>(*a);
     return cudaGetLastError();
 }
 
-// variant: 0 = default (two-row-set kernel), 2 = single-row-set kernel where the bandwidth allows it (measured
-// slower: cartpole 0.399 vs 0.346 ms, car 2.79 vs 2.35 ms -- profiles/kkt_r01_history.jsonl tags v7 / v7two)
-extern "C" int dto_kkt_launch_band(const dto_kkt_args* a, void* stream)
+// W and the half bandwidth -> the <W, BW> instantiation; BW must be the bound dto_kkt_bw_bound gives, which also fixes
+// the layout of the stored factor, so every bound it returns needs a case here
+template <class Kernel>
+static int launch_banded(const dto_kkt_args* a, void* stream)
 {
     if (a->B == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
     cudaError_t e = cudaErrorInvalidValue;
     const int bound = dto_kkt_bw_bound(a->W, a->bw);
-    const bool two = a->variant != 2 || a->virt || a->diag;   // candidate slots / barrier diagonal: default kernel only
     if (a->W == 16) {
-        if (bound == 6) e = two ? launch_band_t<16, 6>(a, st) : launch_band_s<16, 6, 8>(a, st);
-        else if (bound == 9) e = two ? launch_band_t<16, 9>(a, st) : launch_band_s<16, 9, 4>(a, st);
-        else if (bound == 12) e = two ? launch_band_t<16, 12>(a, st) : launch_band_s<16, 12, 4>(a, st);
-        else e = launch_band_t<16, 15>(a, st);
+        if (bound == 6) e = launch_at<Kernel, 16, 6>(a, st);
+        else if (bound == 9) e = launch_at<Kernel, 16, 9>(a, st);
+        else if (bound == 12) e = launch_at<Kernel, 16, 12>(a, st);
+        else e = launch_at<Kernel, 16, 15>(a, st);
     } else if (a->W == 32) {
-        if (bound == 20) e = two ? launch_band_t<32, 20>(a, st) : launch_band_s<32, 20, 8>(a, st);
-        else e = launch_band_t<32, 31>(a, st);
+        if (bound == 20) e = launch_at<Kernel, 32, 20>(a, st);
+        else e = launch_at<Kernel, 32, 31>(a, st);
     }
     return e == cudaSuccess ? 1 : -(int)e;
 }
 
-template <int W, int BW>
-static cudaError_t launch_resolve_t(const dto_kkt_args* a, cudaStream_t st)
-{
-    const int64_t per_block = 4 * (32 / W);
-    if (KktSmem<W, BW>::BYTES > 48 * 1024) {
-        const cudaError_t e = cudaFuncSetAttribute(kkt_resolve_kernel<W, BW>, cudaFuncAttributeMaxDynamicSharedMemorySize, KktSmem<W, BW>::BYTES);
-        if (e != cudaSuccess) return e;
-    }
-    kkt_resolve_kernel<W, BW><<<(unsigned)((a->B + per_block - 1) / per_block), 128, KktSmem<W, BW>::BYTES, st>>>(*a);
-    return cudaGetLastError();
-}
+extern "C" int dto_kkt_launch_band(const dto_kkt_args* a, void* stream) { return launch_banded<BandKernel>(a, stream); }
 
-// forward + backward solve with the stored factor (every factor kernel variant writes the same layout)
-extern "C" int dto_kkt_launch_resolve(const dto_kkt_args* a, void* stream)
-{
-    if (a->B == 0) return 0;
-    cudaStream_t st = (cudaStream_t)stream;
-    cudaError_t e = cudaErrorInvalidValue;
-    const int bound = dto_kkt_bw_bound(a->W, a->bw);
-    if (a->W == 16)
-        e = bound == 6 ? launch_resolve_t<16, 6>(a, st) : bound == 9 ? launch_resolve_t<16, 9>(a, st) : bound == 12 ? launch_resolve_t<16, 12>(a, st)
-                                                                                                                  : launch_resolve_t<16, 15>(a, st);
-    else if (a->W == 32)
-        e = bound == 20 ? launch_resolve_t<32, 20>(a, st) : launch_resolve_t<32, 31>(a, st);
-    return e == cudaSuccess ? 1 : -(int)e;
-}
+// forward + backward solve with the factor the last factor kernel launch stored
+extern "C" int dto_kkt_launch_resolve(const dto_kkt_args* a, void* stream) { return launch_banded<ResolveKernel>(a, stream); }
 
 extern "C" int dto_kkt_launch_assemble(const dto_kkt_args* a, int64_t problem, double* out, void* stream)
 {

@@ -17,9 +17,6 @@ typedef struct dto_kkt_args {
     int32_t W;           /* band entries kept per row = rows per block = lanes per problem (16 or 32) */
     int32_t bw;          /* half bandwidth of the ordered matrix (<= W - 1)                    */
     int32_t nblk;        /* ceil(dim / W) row blocks                                           */
-    int32_t variant;     /* 0: default (two-row-set factor kernel); 2: single-row-set kernel   */
-    int32_t fuse_rhs;    /* 1: the factor kernel computes h = [grad f + J'y ; c] itself (and stores it to rhs) instead of
-                            reading the output of kkt_rhs_kernel: one launch and one pass over h less            */
     int64_t factor_stride; /* doubles of factor storage per problem: nblk*W*LW + nblk*W, LW = dto_kkt_col_width */
     /* callback outputs / inputs of the shard (problem-major) */
     const double* H;     /* [B][nnz_H]  */

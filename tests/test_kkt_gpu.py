@@ -139,7 +139,8 @@ def test_kkt_matches_golden_fixtures():
 
 def test_kkt_full_size_properties():
     """cartpole T=101, B=512: every problem's solution satisfies K x = h to rounding (K rebuilt on the
-    host from the GPU's J, H), results do not depend on sharding, and a second solve is bit-identical."""
+    host from the GPU's J, H), results do not depend on sharding, a second solve is bit-identical, and a
+    solve enqueues two KKT kernels (right-hand side, factor) on top of the callbacks."""
     import scipy.sparse as sp
 
     name, kw, B = "cartpole", dict(T=101), 512
@@ -168,8 +169,14 @@ def test_kkt_full_size_properties():
         worst = max(worst, be)
     assert worst <= 1e-12, f"normwise backward error {worst:.3e}"
     sol2 = np.empty((B, n))
+    l0 = pn.launch_count()
     kkt.solve(sol2)
+    solve_launches = pn.launch_count() - l0
     assert np.array_equal(sol, sol2)
+    l0 = pn.launch_count()
+    kkt.launch(2)                                   # the same callbacks alone
+    pn.sync()
+    assert solve_launches - (pn.launch_count() - l0) == 2
     kkt.close()
     pn.close()
     # two logical shards on the one device: same bits
@@ -214,42 +221,6 @@ def test_kkt_heterogeneous_shape():
         assert np.max(np.abs(Lm @ np.diag(Dv) @ Lm.T - Kp)) <= 1e-13 * np.max(np.abs(Kp)) * growth * 32
         x = sol[b]
         assert np.max(np.abs(Kd @ x - h[b])) <= 1e-13 * growth * (np.linalg.norm(Kd, np.inf) * np.max(np.abs(x)) + np.max(np.abs(h[b])))
-    kkt.close()
-    pn.close()
-
-
-@pytest.mark.parametrize("name,kw,B,config", [("pendulum", dict(), 9, 1), ("cartpole", dict(T=101), 67, 2),
-                                              ("car", dict(T=12, obstacle="general"), 5, 4),
-                                              ("acrobot_hessian_test", dict(), 5, 6)])
-def test_kkt_factor_kernel_variants_agree(name, kw, B, config, monkeypatch):
-    """The two-row-set factor kernel (default) and the single-row-set kernel (DTO_KKT_VARIANT=single, used
-    where the half bandwidth allows it) perform the same operations on the same operands: bit-identical
-    factors and solutions."""
-    mo, osolver, pn, z, lam, sigma, w = _setup(name, kw, B, config)
-    outs = []
-    for variant in ("", "single"):
-        monkeypatch.setenv("DTO_KKT_VARIANT", variant)
-        kkt = PK.KKTSystem(pn)
-        sol = np.empty((B, kkt.dim))
-        l0 = pn.launch_count()
-        kkt.solve(sol, variables=z, scaling=sigma, duals=lam)
-        launches = pn.launch_count() - l0
-        Lm, Dv = kkt.factor(B - 1)
-        outs.append((sol, Lm, Dv))
-        kkt.close()
-    assert np.array_equal(outs[0][2], outs[1][2]) and np.array_equal(outs[0][1], outs[1][1])
-    assert np.array_equal(outs[0][0], outs[1][0])
-    # the FUSE instantiation (DTO_KKT_FUSE_RHS=1: the factor kernel forms h = [g + J'y; c] itself, no kkt_rhs_kernel): the
-    # same additions in the same order, so the same bits -- right-hand side, factor and solution
-    monkeypatch.setenv("DTO_KKT_VARIANT", "")
-    monkeypatch.setenv("DTO_KKT_FUSE_RHS", "1")
-    kkt = PK.KKTSystem(pn)
-    sol = np.empty((B, kkt.dim))
-    l0 = pn.launch_count()
-    kkt.solve(sol, variables=z, scaling=sigma, duals=lam)
-    assert pn.launch_count() - l0 == launches - 1             # the callbacks + ONE KKT kernel instead of two
-    Lm, Dv = kkt.factor(B - 1)
-    assert np.array_equal(sol, outs[0][0]) and np.array_equal(Lm, outs[0][1]) and np.array_equal(Dv, outs[0][2])
     kkt.close()
     pn.close()
 
