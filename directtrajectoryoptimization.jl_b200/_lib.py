@@ -118,6 +118,8 @@ def lib() -> C.CDLL:
         "dto_kkt_analyze_ex": (C.c_int, [vp, C.c_int, i64p, i64p]),
         "dto_hessian_block_count": (i64, [vp]),
         "dto_hessian_block_structure": (C.c_int, [vp, i64p, i64p]),
+        "dto_hessian_chain_count": (i64, [vp]),
+        "dto_hessian_chain_structure": (C.c_int, [vp, i64p, i64p]),
         "dto_kkt_create": (C.c_int, [vp, C.c_double, C.c_double, C.POINTER(vp)]),
         "dto_kkt_create_ex": (C.c_int, [vp, C.c_double, C.c_double, C.c_int, C.POINTER(vp)]),
         "dto_kkt_set_hessian_blocks": (C.c_int, [vp, vp]),

@@ -816,6 +816,54 @@ __device__ __forceinline__ double gsum(double v)
     return v;
 }
 
+// One damped BFGS update of a dense symmetric n x n block (n <= W) held by a group of W lanes, lane i with s_i and y_i of
+// the block's variable i; `upd` is the block's first-update flag. Both quasi-Newton modes call it: k_qn_update on knot
+// blocks, k_pqn_update on element blocks. A lane with i >= n, or a group with `live` false, only takes part in the shuffles.
+template <int W>
+__device__ __forceinline__ void qn_block_update(double* __restrict__ blk, int n, int i, bool live, double s, double y, uint8_t* upd)
+{
+    const bool own = i < n;
+    const double ss = gsum<W>(s * s), sy = gsum<W>(s * y), yy = gsum<W>(y * y);
+    bool ok = live && ss > 1.0e-30 && isfinite(ss) && isfinite(sy) && isfinite(yy);
+    // the block's first update starts from (y'y / s'y) I instead of the identity
+    const bool scale = ok && !*upd && sy > 0.0;
+    const double sc = yy / sy;
+    const int nmax = (int)__reduce_max_sync(FULL, (unsigned)n);
+    double bs = 0.0;   // (B s)_i = sum_j B(j, i) s_j, j ascending
+    for (int j0 = 0; j0 < nmax; j0 += 4) {
+        double v[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) v[u] = (own && j0 + u < n && !scale) ? blk[(j0 + u) * n + i] : 0.0;
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int j = j0 + u;
+            const double sj = __shfl_sync(FULL, s, j & (W - 1), W);
+            if (own && j < n) bs += (scale ? (j == i ? sc : 0.0) : v[u]) * sj;
+        }
+    }
+    const double sBs = gsum<W>(s * bs);
+    const double th = sy >= 0.2 * sBs ? 1.0 : 0.8 * sBs / (sBs - sy);
+    const double r = th * y + (1.0 - th) * bs;
+    const double sr = gsum<W>(s * r);
+    ok = ok && isfinite(sBs) && isfinite(sr) && sBs > 0.0 && sr > 0.0;
+    // B <- B - (Bs)(Bs)'/s'Bs + r r'/s'r: lane i writes column i (bitwise symmetric: both triangles form the same products)
+    for (int j0 = 0; j0 < nmax; j0 += 4) {
+        double v[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) v[u] = (ok && own && j0 + u < n && !scale) ? blk[(j0 + u) * n + i] : 0.0;
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int j = j0 + u;
+            const double bsj = __shfl_sync(FULL, bs, j & (W - 1), W), rj = __shfl_sync(FULL, r, j & (W - 1), W);
+            if (ok && own && j < n) {
+                const double old = scale ? (j == i ? sc : 0.0) : v[u];
+                blk[j * n + i] = old - (bsj * bs) / sBs + (rj * r) / sr;
+            }
+        }
+    }
+    if (ok && i == 0) *upd = 1;
+}
+
 template <int W>
 __global__ void __launch_bounds__(128) k_qn_update(const dto_sqp_args a)
 {
@@ -866,47 +914,110 @@ __global__ void __launch_bounds__(128) k_qn_update(const dto_sqp_args a)
         a.gp[zi] = gn;
     }
     if (a.it == 0) return;   // (uniform over the launch) the previous point is the one just stored
-    const double ss = gsum<W>(s * s), sy = gsum<W>(s * y), yy = gsum<W>(y * y);
-    bool ok = live && ss > 1.0e-30 && isfinite(ss) && isfinite(sy) && isfinite(yy);
-    uint8_t* upd = a.qn_updated + b * a.T + t;
-    // the block's first update starts from (y'y / s'y) I instead of the identity
-    const bool scale = ok && !*upd && sy > 0.0;
-    const double sc = yy / sy;
-    double* __restrict__ blk = a.blocks + b * a.nnz_blk + (live ? a.boff[t] : 0);
-    const int nmax = (int)__reduce_max_sync(FULL, (unsigned)n);
-    double bs = 0.0;   // (B s)_i = sum_j B(j, i) s_j, j ascending
-    for (int j0 = 0; j0 < nmax; j0 += 4) {
-        double v[4];
+    qn_block_update<W>(a.blocks + b * a.nnz_blk + (live ? a.boff[t] : 0), n, i, live, s, y, a.qn_updated + b * a.T + t);
+}
+
+
+// =====================================================================================================================
+// Partitioned damped BFGS (hessian_approximation = 2; sqp.py `PARTITIONED_BFGS` states it): one dense symmetric block B_t
+// per knot element E_t over v_t = [x_t; u_t; x_{t+1}] (the last knot: x_T), a contiguous range of z. A group of W lanes
+// owns one (problem, element), lane i variable i of v_t. s_t = P_t (z - z_prev); y_t = the change of the element's gradient:
+// g + the J'lam terms of the rows of d_t and stage_t on [x_t; u_t], the J'lam terms of d_t's rows on x_{t+1}. The J'lam
+// terms go over the element's own column table (ecolptr/ecolslot/ecolrow, rows ascending), so every J slot has one owning
+// lane, which refreshes J_prev in place as k_qn_update does.
+// The previous point: element t reads z_prev on x_{t+1}, which element t+1 owns and would rewrite in the same launch. So z
+// alternates between two buffers by iteration parity: iteration `it` stores z into buffer it & 1 (owner lanes, i < n_t, only)
+// and reads z_prev from the other one, which no lane writes in this launch. g_prev is read and written on [x_t; u_t] only,
+// by the owner lane.
+// =====================================================================================================================
+template <int W>
+__global__ void __launch_bounds__(128) k_pqn_update(const dto_sqp_args a)
+{
+    const int i = threadIdx.x & (W - 1);
+    const int64_t gid = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / W;   // (problem, element) of this group
+    const bool live = gid < a.B * a.T;
+    const int64_t b = live ? gid / a.T : 0;
+    const int t = live ? (int)(gid - b * a.T) : 0;
+    const int m = live ? a.edim[t] : 0, n = live ? a.kdim[t] : 0;
+    const bool own = i < m;
+    const int zc = a.kofs[t] + i;                                  // variable i of v_t
+    double* __restrict__ blk = a.eblocks + b * a.nnz_el + (live ? a.eoff[t] : 0);
+    double* __restrict__ zcur = (a.it & 1) ? a.zp2 : a.zp;
+    const double* __restrict__ zprev = (a.it & 1) ? a.zp : a.zp2;
+    double s = 0.0, y = 0.0;
+    if (own) {
+        const int64_t zi = b * a.N_z + zc;
+        const double f = a.free[zc];
+        const double zn = a.z[zi], zo = zprev[zi];
+        const double* __restrict__ lam = a.lam + b * a.N_c;
+        const double* __restrict__ Jn = a.bJ + b * a.nnz_J;
+        double* __restrict__ Jo = a.Jp + b * a.nnz_J;
+        double jl = 0.0, jlp = 0.0;
+        const int e = a.evar[t] + i;
+        const int q1 = a.ecolptr[e + 1];
+        for (int q0 = a.ecolptr[e]; q0 < q1; q0 += 4) {
+            int sl[4];
+            double vl[4], vn[4], vo[4];
 #pragma unroll
-        for (int u = 0; u < 4; ++u) v[u] = (own && j0 + u < n && !scale) ? blk[(j0 + u) * n + i] : 0.0;
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int j = j0 + u;
-            const double sj = __shfl_sync(FULL, s, j & (W - 1), W);
-            if (own && j < n) bs += (scale ? (j == i ? sc : 0.0) : v[u]) * sj;
-        }
-    }
-    const double sBs = gsum<W>(s * bs);
-    const double th = sy >= 0.2 * sBs ? 1.0 : 0.8 * sBs / (sBs - sy);
-    const double r = th * y + (1.0 - th) * bs;
-    const double sr = gsum<W>(s * r);
-    ok = ok && isfinite(sBs) && isfinite(sr) && sBs > 0.0 && sr > 0.0;
-    // B <- B - (Bs)(Bs)'/s'Bs + r r'/s'r: lane i writes column i (bitwise symmetric: both triangles form the same products)
-    for (int j0 = 0; j0 < nmax; j0 += 4) {
-        double v[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) v[u] = (ok && own && j0 + u < n && !scale) ? blk[(j0 + u) * n + i] : 0.0;
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int j = j0 + u;
-            const double bsj = __shfl_sync(FULL, bs, j & (W - 1), W), rj = __shfl_sync(FULL, r, j & (W - 1), W);
-            if (ok && own && j < n) {
-                const double old = scale ? (j == i ? sc : 0.0) : v[u];
-                blk[j * n + i] = old - (bsj * bs) / sBs + (rj * r) / sr;
+            for (int u = 0; u < 4; ++u) {
+                const bool in = q0 + u < q1;
+                sl[u] = in ? a.ecolslot[q0 + u] : 0;
+                vl[u] = in ? lam[a.ecolrow[q0 + u]] : 0.0;
             }
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                vn[u] = q0 + u < q1 ? Jn[sl[u]] : 0.0;
+                vo[u] = q0 + u < q1 ? Jo[sl[u]] : 0.0;
+            }
+#pragma unroll
+            for (int u = 0; u < 4; ++u)
+                if (q0 + u < q1) {
+                    jl += vn[u] * vl[u];
+                    jlp += vo[u] * vl[u];
+                    Jo[sl[u]] = vn[u];
+                }
+        }
+        s = (zn - zo) * f;
+        if (i < n) {   // [x_t; u_t]: the cost's gradient too; these lanes own z_prev and g_prev of their variable
+            const double gn = a.bg[zi], go = a.gp[zi];
+            y = ((gn + jl) - (go + jlp)) * f;
+            zcur[zi] = zn;
+            a.gp[zi] = gn;
+        } else {
+            y = (jl - jlp) * f;
         }
     }
-    if (ok && i == 0) *upd = 1;
+    if (a.it == 0) {   // (uniform over the launch) every solve and continuation stage starts from identity element blocks
+        if (own)
+            for (int j = 0; j < m; ++j) blk[j * m + i] = j == i ? 1.0 : 0.0;
+        return;
+    }
+    qn_block_update<W>(blk, m, i, live, s, y, a.qn_updated + b * a.T + t);
+}
+
+// H of K from the element blocks: chain row block t (rows [x_t; u_t], columns [x_t; u_t; x_{t+1}], dense row-major) is
+// B_t[0:n_t, :], plus the x_t x x_t tail of B_{t-1} on its x_t x x_t corner (in that order: sqp.py sums the same way).
+// Lane j writes column j; no two groups write the same entry.
+template <int W>
+__global__ void __launch_bounds__(128) k_pqn_assemble(const dto_sqp_args a)
+{
+    const int j = threadIdx.x & (W - 1);
+    const int64_t gid = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) / W;
+    if (gid >= a.B * a.T) return;
+    const int64_t b = gid / a.T;
+    const int t = (int)(gid - b * a.T);
+    const int m = a.edim[t], n = a.kdim[t];
+    if (j >= m) return;
+    const double* __restrict__ E = a.eblocks + b * a.nnz_el + a.eoff[t];
+    double* __restrict__ C = a.blocks + b * a.nnz_blk + a.boff[t];
+    const int mp = t > 0 ? a.edim[t - 1] : 0, np = t > 0 ? a.kdim[t - 1] : 0;
+    const int nx = mp - np;                                        // x_t: the tail of element t - 1
+    const double* __restrict__ P = a.eblocks + b * a.nnz_el + (t > 0 ? a.eoff[t - 1] + np * mp + np : 0);
+    for (int r = 0; r < n; ++r) {
+        double v = E[r * m + j];
+        if (r < nx && j < nx) v += P[r * mp + j];
+        C[r * m + j] = v;
+    }
 }
 
 template <class K, class... Args>
@@ -969,6 +1080,30 @@ extern "C" int dto_sqp_k_qn_update(const dto_sqp_args* a, void* s)
         k_qn_update<16><<<grid, 128, 0, (cudaStream_t)s>>>(*a);
     else
         k_qn_update<32><<<grid, 128, 0, (cudaStream_t)s>>>(*a);
+    const cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : -(int)e;
+}
+extern "C" int dto_sqp_k_pqn_update(const dto_sqp_args* a, void* s)
+{
+    const int64_t threads = a->B * a->T * a->qn_W;
+    if (threads <= 0) return 0;
+    const unsigned grid = (unsigned)((threads + 127) / 128);
+    if (a->qn_W == 16)
+        k_pqn_update<16><<<grid, 128, 0, (cudaStream_t)s>>>(*a);
+    else
+        k_pqn_update<32><<<grid, 128, 0, (cudaStream_t)s>>>(*a);
+    const cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? 0 : -(int)e;
+}
+extern "C" int dto_sqp_k_pqn_assemble(const dto_sqp_args* a, void* s)
+{
+    const int64_t threads = a->B * a->T * a->qn_W;
+    if (threads <= 0) return 0;
+    const unsigned grid = (unsigned)((threads + 127) / 128);
+    if (a->qn_W == 16)
+        k_pqn_assemble<16><<<grid, 128, 0, (cudaStream_t)s>>>(*a);
+    else
+        k_pqn_assemble<32><<<grid, 128, 0, (cudaStream_t)s>>>(*a);
     const cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? 0 : -(int)e;
 }

@@ -85,6 +85,16 @@ typedef struct dto_sqp_args {
     const int32_t *colptr, *colslot, *colrow;   /* the KKT handle's Jacobian-by-column tables (J'lam, rows ascending) */
     double *zp, *gp, *Jp;                  /* z, g, J of the previous iteration                                */
     uint8_t* qn_updated;                   /* [B][T] 1 once a block has taken an update (the first one is scaled) */
+    /* partitioned damped BFGS (hessian_approximation = 2): element t covers z[kofs[t], kofs[t] + edim[t]) = [x_t; u_t; x_{t+1}]
+     * (the last knot: x_T) and is a dense row-major edim[t]^2 matrix at offset eoff[t] of the problem's nnz_el element values;
+     * T, qn_W, kofs, kdim (= n_t), bJ, Jp, gp and qn_updated (one flag per element) as above; blocks / nnz_blk / boff: the KKT
+     * handle's chain array, row block t (kdim[t] x edim[t]) at offset boff[t] */
+    const int32_t *edim, *eoff, *evar;     /* [T]; evar[t] = sum_{s<t} edim[s]: element t's first entry of ecolptr         */
+    int32_t nnz_el;
+    double* eblocks;                       /* [B][nnz_el]                                                       */
+    const int32_t *ecolptr, *ecolslot, *ecolrow;   /* [sum_t edim[t] + 1], [nnz_J], [nnz_J]: J entries of the rows of d_t and
+                                                      stage_t by variable of v_t, rows ascending                     */
+    double* zp2;                           /* [B][N_z] z_prev of odd iterations (zp: even ones)                 */
 } dto_sqp_args;
 
 /* each returns 0 or -(cudaError_t) */
@@ -110,6 +120,11 @@ int dto_sqp_k_ip_ls_round(const dto_sqp_args* a, int32_t round, void* stream);
 int dto_sqp_k_ip_end(const dto_sqp_args* a, void* stream);
 /* knot-block damped BFGS: update every block from s = z - zp, y = (g + J'lam) - (gp + Jp'lam), then zp, gp, Jp = z, g, J */
 int dto_sqp_k_qn_update(const dto_sqp_args* a, void* stream);
+/* partitioned damped BFGS: update every element block from its s_t, y_t (identity element blocks at it = 0), then z, g, J
+ * become the previous ones */
+int dto_sqp_k_pqn_update(const dto_sqp_args* a, void* stream);
+/* chain row blocks (H of K) from the element blocks */
+int dto_sqp_k_pqn_assemble(const dto_sqp_args* a, void* stream);
 /* slot k * R + j (k-th entry of oidx, j < R) <- z + alpha 2^-j dz and the problem's parameters */
 int dto_sqp_k_multi_trial(const dto_sqp_args* a, int32_t count, int32_t R, void* stream);
 /* per open problem: the first j whose trial passes the Armijo test is taken, as R sequential rounds would */

@@ -86,6 +86,7 @@ class BatchedNLPData:
         self.batch = int(batch)
         self.devices = list(devices) if devices is not None else None
         self.hessian_lagrangian = bool(evaluate_hessian)
+        self.use_general = bool(use_general)
         self._keep = [_i32(dynamics_kind), _i32(cost_kind), _i32(stage_kind), _i32(parameter_dim),
                       _i32(parameter_offset) if parameter_offset is not None else None]
         ip = C.POINTER(C.c_int32)
@@ -133,6 +134,17 @@ class BatchedNLPData:
         r = np.empty(n, dtype=np.int64)
         c = np.empty(n, dtype=np.int64)
         _lib.check(_lib.lib().dto_hessian_block_structure(self.shape, r.ctypes.data_as(C.POINTER(C.c_int64)),
+                                                          c.ctypes.data_as(C.POINTER(C.c_int64))))
+        return r, c
+
+    def hessian_chain_structure(self):
+        """(rows, cols), 1-based, sorted: row block t of the knot chain, rows [x_t; u_t] against columns [x_t; u_t; x_{t+1}]
+        (the last knot: x_T against x_T), dense row-major. The H of a KKT system in knot-chain mode, e.g. the solver's
+        partitioned BFGS approximation (sqp.py `PARTITIONED_BFGS`)."""
+        n = int(_lib.lib().dto_hessian_chain_count(self.shape))
+        r = np.empty(n, dtype=np.int64)
+        c = np.empty(n, dtype=np.int64)
+        _lib.check(_lib.lib().dto_hessian_chain_structure(self.shape, r.ctypes.data_as(C.POINTER(C.c_int64)),
                                                           c.ctypes.data_as(C.POINTER(C.c_int64))))
         return r, c
 
@@ -442,8 +454,8 @@ class Solver:
             clo, cup = self.nlp.constraint_bounds
             pinned = np.isfinite(lo) & (lo == up)
             rows_ok = bool(np.all((clo == cup) | (np.isneginf(clo) & (cup == 0.0))))      # equalities and c(z) <= 0 rows
-            # a problem without Hessians reaches the native solver when its knot-block BFGS mode is asked for
-            qn = (options or {}).get("hessian_approximation", "exact") == "knot-bfgs"
+            # a problem without Hessians reaches the native solver when one of its quasi-Newton modes is asked for
+            qn = (options or {}).get("hessian_approximation", "exact") in ("knot-bfgs", "partitioned-bfgs")
             ok = (self.nlp.hessian_lagrangian or qn) and rows_ok        # (several devices: one native solve per device, side by side)
             # (bounds on variables (Bound(action_lower = ..., ...)) and inequality rows (Constraint(...; indices_inequality)): the
             # interior-point mode, in both arms)

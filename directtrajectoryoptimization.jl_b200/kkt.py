@@ -20,7 +20,7 @@ from . import _lib
 from .evaluator import BatchedNLPData, _out, _p
 
 
-HESSIAN = {"exact": 0, "knot-blocks": 1}   # DTO_KKT_HESSIAN_EXACT, DTO_KKT_HESSIAN_KNOT_BLOCKS
+HESSIAN = {"exact": 0, "knot-blocks": 1, "knot-chain": 2}   # DTO_KKT_HESSIAN_EXACT, _KNOT_BLOCKS, _KNOT_CHAIN
 
 
 def _hessian_mode(hessian: str) -> int:
@@ -32,7 +32,8 @@ def _hessian_mode(hessian: str) -> int:
 def analyze(nlp: BatchedNLPData, hessian: str = "exact"):
     """Host-only symbolic phase: (perm, bandwidth). perm[p] is the 1-based index (variables first,
     then constraint rows) placed at position p of the banded ordering. hessian="knot-blocks": the H block
-    of K is one dense block per knot (nlp.hessian_block_structure()) instead of the Hessian's structure."""
+    of K is one dense block per knot (nlp.hessian_block_structure()) instead of the Hessian's structure; hessian="knot-chain":
+    one row block per knot over [x_t; u_t] x [x_t; u_t; x_{t+1}] (nlp.hessian_chain_structure())."""
     n = nlp.num_variables + nlp.num_constraint
     perm = np.empty(n, dtype=np.int64)
     bw = C.c_int64()
@@ -46,7 +47,8 @@ class KKTSystem:
     hessian="knot-blocks": H is not the callbacks' Hessian but one dense symmetric block per knot owned by this
     object (the identity at first; set_hessian_blocks / hessian_blocks, shape [B, nnz_blk] in the order of
     nlp.hessian_block_structure()); the callbacks then run without a Hessian pass, so a problem built without
-    evaluate_hessian works."""
+    evaluate_hessian works. hessian="knot-chain": the same with H = the chain of nlp.hessian_chain_structure(), [B, nnz_chain]
+    (row block t: rows [x_t; u_t], columns [x_t; u_t; x_{t+1}], dense row-major; the identity at first)."""
 
     def __init__(self, nlp: BatchedNLPData, primal_reg: float = 1.0e-5, dual_reg: float = 1.0e-5, hessian: str = "exact"):
         L = _lib.lib()
@@ -55,7 +57,8 @@ class KKTSystem:
         h = C.c_void_p()
         _lib.check(L.dto_kkt_create_ex(nlp.handle, float(primal_reg), float(dual_reg), _hessian_mode(hessian), C.byref(h)))
         self._h = h
-        self.num_blocks = int(L.dto_hessian_block_count(nlp.shape)) if hessian == "knot-blocks" else 0
+        self.num_blocks = {"knot-blocks": lambda: int(L.dto_hessian_block_count(nlp.shape)),
+                           "knot-chain": lambda: int(L.dto_hessian_chain_count(nlp.shape))}.get(hessian, lambda: 0)()
         self.dim = int(L.dto_kkt_dim(h))
         self.bandwidth = int(L.dto_kkt_bandwidth(h))
         self.row_width = int(L.dto_kkt_row_width(h))
@@ -162,13 +165,13 @@ class KKTSystem:
         return Lm, D
 
     def set_hessian_blocks(self, blocks) -> None:
-        """knot-blocks mode: the blocks of every problem, [B, nnz_blk] (host -> device)."""
+        """knot-blocks / knot-chain mode: the blocks (the chain) of every problem, [B, nnz_blk] (host -> device)."""
         from .evaluator import _f64
         v = _f64(blocks, (self.nlp.batch, self.num_blocks), "blocks")
         _lib.check(_lib.lib().dto_kkt_set_hessian_blocks(self._h, _p(v)))
 
     def hessian_blocks(self) -> np.ndarray:
-        """knot-blocks mode: the blocks of every problem, [B, nnz_blk] (device -> host)."""
+        """knot-blocks / knot-chain mode: the blocks (the chain) of every problem, [B, nnz_blk] (device -> host)."""
         out = np.empty((self.nlp.batch, self.num_blocks))
         _lib.check(_lib.lib().dto_kkt_get_hessian_blocks(self._h, _p(out)))
         return out

@@ -45,9 +45,9 @@ from typing import Optional
 
 
 class HessianApproximation(str):
-    """"exact" or "knot-bfgs": a str whose float() is its dto_sqp_options.hessian_approximation code"""
+    """"exact", "knot-bfgs" or "partitioned-bfgs": a str whose float() is its dto_sqp_options.hessian_approximation code"""
 
-    CODES = {"exact": 0, "knot-bfgs": 1}
+    CODES = {"exact": 0, "knot-bfgs": 1, "partitioned-bfgs": 2}
 
     def __float__(self):
         return float(self.CODES[str(self)])
@@ -103,7 +103,9 @@ class SQPOptions:
                                        #   widened about their midpoint by this factor, solved, then the true bounds warm-started (<= 1: off)
     hessian_approximation: str = HessianApproximation("exact")   # "knot-bfgs": H is one dense block per knot, updated by damped BFGS (`knot_bfgs_update`) --
                                        #   for problems built without Hessians (the reference's default evaluate_hessian = false);
-                                       #   the native arm only. exact_below does not apply (H is always the blocks)
+                                       #   the native arm only. exact_below does not apply (H is always the blocks).
+                                       #   "partitioned-bfgs": one damped BFGS block per knot element over [x_t; u_t; x_{t+1}]
+                                       #   (`knot_elements` states it); no general constraint
 
 
 class SQPResult:
@@ -421,6 +423,72 @@ def knot_bfgs_update(xp, blocks, s, y, free, first):
     dBs, dsr = xp.where(ok, sBs, one), xp.where(ok, sr, one)
     Bn = B0 - (Bs[:, :, None] * Bs[:, None, :]) / dBs[:, None, None] + (r[:, :, None] * r[:, None, :]) / dsr[:, None, None]
     return xp.where(ok[:, None, None], Bn, blocks), first & ~ok
+
+
+def knot_elements(nlp):
+    """The partitioned damped BFGS approximation ("partitioned-bfgs", dto_sqp_options.hessian_approximation = 2). Stated here
+    once; dto_sqp.cu `k_pqn_update` / `k_pqn_assemble`, the KKT layer's knot chain (DTO_KKT_HESSIAN_KNOT_CHAIN) and the tests'
+    twin follow it.
+
+    The Lagrangian L = sigma f + lam'c splits into one element per knot t = 0..T-1 (0-based; sigma, lam as the solver holds them):
+      t < T-1:  E_t(x_t, u_t, x_{t+1}) = sigma cost_t(x_t, u_t) + lam_{S,t}' stage_t(x_t, u_t) + lam_{D,t}' d_t(x_{t+1}, x_t, u_t)
+      t = T-1:  E_t(x_T) = sigma cost_T(x_T) + lam_{S,T}' stage_T(x_T)
+    Element t's variables v_t = [x_t; u_t; x_{t+1}] are one contiguous range z[v0_t, v0_t + m_t), m_t = n_t + nx_{t+1}
+    (n_t = nx_t + nu_t; the last knot: m = n = nx_T). Without a general constraint sum_t E_t = L, so the Hessian of L is
+    sum_t P_t' (Hessian of E_t) P_t. Each element keeps a dense symmetric m_t x m_t block B_t (the identity at the start of
+    every solve and continuation stage); after the callbacks of every iteration (where "knot-bfgs" updates its blocks)
+      s_t = P_t (z - z_prev), pinned variables masked;
+      y_t = grad_{v_t} E_t(z) - grad_{v_t} E_t(z_prev), both with the multipliers as they stand (bound multipliers left out):
+            on [x_t; u_t] g (only cost_t touches them in the objective) + the J'lam terms of the rows of d_t and stage_t,
+            on x_{t+1} the J'lam terms of the rows of d_t only (`element_gradients`);
+    and B_t takes exactly the update `knot_bfgs_update` states (first update scaled, Powell damping, the same skips).
+    H of K is sum_t P_t' B_t P_t, kept as the knot chain: row block t = B_t[0:n_t, :] plus, on its x_t x x_t corner, the
+    x_t x x_t tail of B_{t-1}, added in that order (`chain_from_elements`).
+
+    Returns [(v0, n, m, rows)] per knot: 0-based first variable, n_t, m_t, and the constraint rows of d_t and stage_t (0-based,
+    ascending; the rows of J that element t owns). A shape with a general constraint has none: ValueError."""
+    import numpy as np
+    if getattr(nlp, "use_general", False):
+        raise ValueError("partitioned BFGS: a general constraint couples distant knots; no knot element owns its curvature")
+    xs, nx, _, nu = nlp.knot_layout()
+    T = int(nlp.T)
+    jr, jc = (np.asarray(v) - 1 for v in nlp.jacobian_structure_arrays())
+    n_dyn = int(sum(int(nx[t + 1]) for t in range(T - 1)))      # d_t has nx_{t+1} rows; all dynamics rows come first
+    out, r0 = [], 0
+    for t in range(T):
+        v0, n = int(xs[t]) - 1, int(nx[t] + nu[t])
+        m = n + (int(nx[t + 1]) if t + 1 < T else 0)
+        dyn = list(range(r0, r0 + (m - n)))
+        r0 += m - n
+        stage = np.unique(jr[(jr >= n_dyn) & (jc >= v0) & (jc < v0 + n)]).tolist()
+        out.append((v0, n, m, np.array(dyn + stage, dtype=np.int64)))
+    return out
+
+
+def element_gradients(elements, g, Jd, lam):
+    """numpy: grad_{v_t} E_t of every element (`knot_elements`), [B, m_t] each, from g [B, N_z], the dense Jacobian Jd
+    [B, N_c, N_z] and lam [B, N_c]"""
+    import numpy as np
+    out = []
+    for v0, n, m, rows in elements:
+        gr = np.einsum("brj,br->bj", Jd[:, rows, v0:v0 + m], lam[:, rows])
+        gr[:, :n] += g[:, v0:v0 + n]
+        out.append(gr)
+    return out
+
+
+def chain_from_elements(elements, blocks):
+    """numpy: the knot chain [B, nnz_chain] (nlp.hessian_chain_structure() order) from the element blocks [B, m_t, m_t]"""
+    import numpy as np
+    rows = []
+    for t, (v0, n, m, _) in enumerate(elements):
+        top = blocks[t][:, :n, :].copy()
+        if t > 0:
+            npv = elements[t - 1][1]                        # B_{t-1}'s tail: its x_t x x_t corner
+            k = elements[t - 1][2] - npv
+            top[:, :k, :k] = top[:, :k, :k] + blocks[t - 1][:, npv:, npv:]
+        rows.append(top.reshape(top.shape[0], -1))
+    return np.concatenate(rows, axis=1)
 
 
 def bound_arrays(lo, up, options: Optional[SQPOptions] = None, clo=None, cup=None, scale: float = 1.0):

@@ -194,20 +194,30 @@ int dto_kkt_analyze(const dto_shape* s, int64_t* perm, int64_t* bandwidth);
  * n_t x n_t matrix, n_t = nx_t + nu_t, at offset sum_{s<t} n_s^2 of a problem's nnz_blk = sum_t n_t^2 values. */
 #define DTO_KKT_HESSIAN_EXACT 0
 #define DTO_KKT_HESSIAN_KNOT_BLOCKS 1
+/* KNOT_CHAIN: one row block per knot, owned by the KKT handle like KNOT_BLOCKS, that couples neighbouring knots: row block t has
+ * rows [x_t; u_t] and columns [x_t; u_t; x_{t+1}] (the last knot: x_T against x_T) and is a dense row-major n_t x m_t matrix,
+ * m_t = n_t + nx_{t+1}, at offset sum_{s<t} n_s m_s of a problem's nnz_chain = sum_t n_t m_t values. Its first n_t columns are
+ * a symmetric block (both triangles listed); the x_{t+1} columns are the upper copy of the coupling (row < col). The solver's
+ * partitioned BFGS mode (hessian_approximation = 2) keeps H in this form. */
+#define DTO_KKT_HESSIAN_KNOT_CHAIN 2
 /* nnz_blk, and the (row, col) of every block entry, 1-based, sorted (both triangles, like dto_hessian_lagrangian_structure) */
 int64_t dto_hessian_block_count(const dto_shape* s);
 int dto_hessian_block_structure(const dto_shape* s, int64_t* rows, int64_t* cols);
-/* dto_kkt_analyze for either Hessian structure; KNOT_BLOCKS fails with DTO_ERR_UNSUPPORTED when a knot has more than 32
- * variables or the ordered half bandwidth exceeds 31 */
+/* nnz_chain, and the (row, col) of every chain entry, 1-based, sorted (host-only) */
+int64_t dto_hessian_chain_count(const dto_shape* s);
+int dto_hessian_chain_structure(const dto_shape* s, int64_t* rows, int64_t* cols);
+/* dto_kkt_analyze for any Hessian structure; KNOT_BLOCKS fails with DTO_ERR_UNSUPPORTED when a knot has more than 32
+ * variables, KNOT_CHAIN when an element [x_t; u_t; x_{t+1}] has more than 32, and both when the ordered half bandwidth
+ * exceeds 31 */
 int dto_kkt_analyze_ex(const dto_shape* s, int hessian, int64_t* perm, int64_t* bandwidth);
 /* fails with DTO_ERR_UNSUPPORTED when the ordered half bandwidth exceeds 31. The handle borrows the
  * batch: destroy it BEFORE dto_batch_destroy(b); like the batch it is used from one host thread at a time. */
 int dto_kkt_create(dto_batch* b, double primal_reg, double dual_reg, dto_kkt** out);
-/* dto_kkt_create(...) = dto_kkt_create_ex(..., DTO_KKT_HESSIAN_EXACT, ...). With KNOT_BLOCKS the handle owns the blocks
- * [B][nnz_blk] (the identity at creation), the shape needs no Hessian, and every callback pass below evaluates the gradient,
- * the constraints and the Jacobian only (no Hessian pass). */
+/* dto_kkt_create(...) = dto_kkt_create_ex(..., DTO_KKT_HESSIAN_EXACT, ...). With KNOT_BLOCKS (KNOT_CHAIN) the handle owns the
+ * blocks [B][nnz_blk] (the chain [B][nnz_chain]), the identity at creation, the shape needs no Hessian, and every callback pass
+ * below evaluates the gradient, the constraints and the Jacobian only (no Hessian pass). */
 int dto_kkt_create_ex(dto_batch* b, double primal_reg, double dual_reg, int hessian, dto_kkt** out);
-/* host <-> device copies of the knot blocks, [B][nnz_blk] (KNOT_BLOCKS handles only) */
+/* host <-> device copies of the knot blocks, [B][nnz_blk], or of the chain, [B][nnz_chain] (KNOT_BLOCKS / KNOT_CHAIN handles) */
 int dto_kkt_set_hessian_blocks(dto_kkt* k, const double* blocks);
 int dto_kkt_get_hessian_blocks(dto_kkt* k, double* blocks);
 void dto_kkt_destroy(dto_kkt* k);
@@ -261,7 +271,7 @@ int dto_kkt_factor(dto_kkt* k, int64_t problem, double* Lband, double* D);
  * 5 a per-problem diagonal [shard size][dim] (natural order: variables, then constraint rows) ADDED to K from then on (zero
  * at first: the barrier terms of an interior-point solver -- z_L / (x - l) + z_U / (u - x) on variables with Bound(...),
  * src/bounds.jl; -t_i / lambda_i on inequality rows, Constraint(...; indices_inequality), src/constraints.jl), 6 the knot blocks
- * [shard size][nnz_blk] (KNOT_BLOCKS handles only) */
+ * [shard size][nnz_blk] or the chain [shard size][nnz_chain] (KNOT_BLOCKS / KNOT_CHAIN handles only) */
 void* dto_kkt_device_pointer(dto_kkt* k, int which, int shard);
 
 /* ---- batched solver: the caller of the callback path (SURVEY 8f N1) ----
@@ -297,7 +307,10 @@ typedef struct dto_sqp_options {
                                 the true bounds warm-started from there (<= 1: no such fallback) */
     int32_t hessian_approximation;   /* 0: the exact Hessian of the Lagrangian (needs evaluate_hessian); 1: knot-block damped BFGS
                                         (no Hessian needed: one dense block per knot, updated once per iteration from the change of
-                                        the Lagrangian's gradient; Nocedal & Wright, Procedure 18.2) */
+                                        the Lagrangian's gradient; Nocedal & Wright, Procedure 18.2); 2: partitioned damped BFGS
+                                        (no Hessian needed: one dense block per knot element over [x_t; u_t; x_{t+1}], updated from
+                                        the change of that element's gradient -- cost, stage constraint and dynamics d_t -- and
+                                        summed into a KNOT_CHAIN H; a shape with a general constraint -> DTO_ERR_UNSUPPORTED) */
 } dto_sqp_options;
 void dto_sqp_default_options(dto_sqp_options* o);
 /* Solves every problem of a one-shard batch (several devices: one batch and one host thread per device) from z0 [B][N_z] (lambda0 [B][N_c] or NULL = 0). lower / upper [N_z] or

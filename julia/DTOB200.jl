@@ -399,7 +399,8 @@ Base.@kwdef struct SQPOptions
     mu_init::Float64 = 0.1;  barrier_kappa_eps::Float64 = 10.0;  barrier_kappa_mu::Float64 = 0.2;  barrier_theta_mu::Float64 = 1.5
     tau_min::Float64 = 0.99;  bound_push::Float64 = 1.0e-2;  bound_frac::Float64 = 1.0e-2;  kappa_sigma::Float64 = 1.0e10
     tiny_step::Float64 = 1.0e-6;  bound_relax::Float64 = 10.0
-    hessian_approximation::Int32 = 0      # 0 exact Hessian, 1 knot-block damped BFGS (problems built with evaluate_hessian = false)
+    hessian_approximation::Int32 = 0      # 0 exact Hessian, 1 knot-block damped BFGS, 2 partitioned damped BFGS (problems built
+                                          # with evaluate_hessian = false; 2: one block per knot element over [x_t; u_t; x_{t+1}])
 end
 
 """
@@ -430,13 +431,15 @@ function solve_batch(nlp::BatchedNLPData, z0::Matrix{Float64}; lower=nothing, up
     (z=z, lambda=lam, iterations=Int.(its), converged=conv .!= 0, constraint_violation=cv, dual_residual=dr, objective=f, stats=stats)
 end
 
-# hessian_approximation = :knot_bfgs solves a batch built without Hessians (the reference's default evaluate_hessian = false,
-# which puts Ipopt in its limited-memory quasi-Newton mode) with the native solver's knot-block damped BFGS
+# hessian_approximation = :knot_bfgs or :partitioned_bfgs solves a batch built without Hessians (the reference's default
+# evaluate_hessian = false, which puts Ipopt in its limited-memory quasi-Newton mode) with the native solver's knot-block or
+# partitioned (knot elements over [x_t; u_t; x_{t+1}]; no general constraint) damped BFGS
 function DTO.solve!(solver::Solver; hessian_approximation::Symbol=:exact)
     size(solver.z0, 2) == 1 && return MOI.optimize!(solver.optimizer)
-    hessian_approximation in (:exact, :knot_bfgs) || throw(ArgumentError("hessian_approximation must be :exact or :knot_bfgs"))
+    codes = Dict(:exact => Int32(0), :knot_bfgs => Int32(1), :partitioned_bfgs => Int32(2))
+    haskey(codes, hessian_approximation) || throw(ArgumentError("hessian_approximation must be :exact, :knot_bfgs or :partitioned_bfgs"))
     max_iter = Int32(get(solver.optimizer.options, "max_iter", 200))               # Options.max_iter (src/options.jl:9)
-    options = SQPOptions(max_iter=max_iter, hessian_approximation=Int32(hessian_approximation === :knot_bfgs))
+    options = SQPOptions(max_iter=max_iter, hessian_approximation=codes[hessian_approximation])
     solve_batch(solver.nlp, solver.z0; lower=solver.lower, upper=solver.upper, options=options)
 end
 "the last z any callback was handed (the reference returns its internal per-knot buffers, src/solver.jl:41-43)"
