@@ -341,8 +341,8 @@ __global__ void __launch_bounds__((DTO_WS_COMPUTE + DTO_WS_HELPERS) * 32, 1) kno
     const int T = a.T;
     const int total = (int)(a.B * T);
     const int tiles = (total + OWN - 1) / OWN;
-    // programmatic dependent launch: the next kernel of the stream may start its CTAs as soon as SMs free up
-    // (its own prologue then overlaps this grid's tail); it waits in griddepcontrol.wait before touching data
+    // programmatic dependent launch: the next kernel of the stream may start its CTAs as soon as SMs free up, and
+    // load and compute its first tiles while this grid finishes (see launch_pdl for what it may do before its wait)
     asm volatile("griddepcontrol.launch_dependents;");
 
     // the knot table lives in shared memory (the launch plan guarantees it fits). Only the slow path (ragged last
@@ -375,9 +375,11 @@ __global__ void __launch_bounds__((DTO_WS_COMPUTE + DTO_WS_HELPERS) * 32, 1) kno
     const int4* __restrict__ plan = reinterpret_cast<const int4*>(a.ws_plan);
     const int G4 = ws_gen_int4<MODE>(a);  // int4 of general-constraint records per plan block / stage
 
-    // everything up to here touched only shared memory and launch-constant tables; problem data (z, lambda, sigma,
-    // w, outputs) may still be in use by the previous kernel of the stream until it has completed: each role
-    // executes griddepcontrol.wait right before its first access to problem data
+    // The previous kernel of the stream may still be running. It writes none of what this kernel reads (z, lambda,
+    // sigma, w, the knot and plan tables: see launch_pdl), but it may still write, or not yet have written, g, c, J
+    // and H. So only global WRITES wait for it: a helper executes griddepcontrol.wait before its first store, and
+    // the compute warps, which write shared memory only, never wait. Helper 0 of CTA 0 always drains tile 0, so
+    // this grid does not complete before the previous one has (and a later launch's wait covers both).
     if (warp < DTO_WS_HELPERS) {
         // =============================== helper warp ===============================
         asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(DTO_WS_HREG));
@@ -402,6 +404,10 @@ __global__ void __launch_bounds__((DTO_WS_COMPUTE + DTO_WS_HELPERS) * 32, 1) kno
                 int4* sdesc = reinterpret_cast<int4*>(smc + 8 + din + in_sz);   // d0[32] d1[32] d2[32] piece[32] header
                 const int od = (kk - 2) & (NOUT - 1), nd = (kk - 2) >> (NOUT - 1);  // output buffer / use count of tile kk-2 (NOUT is 1 or 2)
                 if (have_drain) {
+                    if (!dep_ok) {   // first global write of this warp: wait until the previous kernel has completed
+                        asm volatile("griddepcontrol.wait;" ::: "memory");
+                        dep_ok = true;
+                    }
                     // ---- tile kk-2 is complete in output buffer od: issue its stores (piece list of stage st)
                     mbar_wait(bar0 + 16 + od * 8, nd & 1);
                     const int4 pd = sdesc[96 + lane];
@@ -454,10 +460,6 @@ __global__ void __launch_bounds__((DTO_WS_COMPUTE + DTO_WS_HELPERS) * 32, 1) kno
                         sdesc[96 + lane] = piece;
                         if (G4) reinterpret_cast<int*>(sdesc + 128 + 32 * DTO_WS_GEN_K)[lane] = -1;  // general entries: table path
                     }
-                    if (!dep_ok) {   // the plan records of the first tile were fetched while the previous kernel drained
-                        asm volatile("griddepcontrol.wait;" ::: "memory");
-                        dep_ok = true;
-                    }
                     if (copy.y > 0) {
                         mbar_expect_tx(full, (uint32_t)copy.y);
                         bulk_load(smem_u32(smc + copy.z + din), ws_in_array(a, copy.w, b0) + copy.x, (uint32_t)copy.y, full);
@@ -481,7 +483,6 @@ __global__ void __launch_bounds__((DTO_WS_COMPUTE + DTO_WS_HELPERS) * 32, 1) kno
     } else {
         // =============================== compute warp ===============================
         asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(DTO_WS_CREG));
-        asm volatile("griddepcontrol.wait;" ::: "memory");   // (parameters not staged in shared memory are read from HBM)
         const int c = warp - DTO_WS_HELPERS;
         double* __restrict__ smc = dto_smem + kt_doubles + (size_t)c * per_warp;
         const uint32_t bar0 = smem_u32(smc);

@@ -819,7 +819,12 @@ inline int plan_persistent(dto_launch_args& b, int64_t* smem_out, int min_ops_ok
 }
 
 // launch with programmatic stream serialization: the kernel may be scheduled while the previous kernel of the stream
-// drains; it must execute griddepcontrol.wait before touching anything that kernel may still read or write
+// drains. A kernel launched here may read, before griddepcontrol.wait, anything that no kernel launched here writes.
+// It must execute the wait before its first global write.
+// The kernels launched here (knot_kernel, knot_kernel_ws) write only g, c, J and H. z, lambda, sigma, w, the knot
+// table and the plan table are written only by copies and by kernels that do not execute launch_dependents, so such
+// a writer has completed before any later kernel launched here starts, also along a chain of launches made here.
+// knot_kernel waits at its top; knot_kernel_ws reads and computes first and waits before its first store.
 template <class K>
 inline cudaError_t launch_pdl(K kernel, unsigned grid, unsigned block, size_t smem, cudaStream_t st, const dto_launch_args& args)
 {
