@@ -45,8 +45,10 @@ __device__ __forceinline__ void row_copy(double* __restrict__ dst, const double*
         st4(dst, i, n, v);
     }
 }
-// dst = x + alpha * y (alpha is 1, -1 or a power of two in every caller: the product is exact, fused or not). dst may
-// be x or y (in-place updates): the four loads of a batch precede its stores in program order, nothing is restrict here
+// dst = x + alpha * y. dst may be x or y (in-place updates): the four loads of a batch precede its stores in program order,
+// nothing is restrict here. The equality-mode callers pass 1, -1 or a power of two, where the product is exact, fused or not;
+// k_ip_ls_round passes amax * 2^-k, where a contraction to an FMA rounds once and a separate multiply and add round twice, so
+// its trial point may differ from the twin's z + alpha * dz in the last bit
 __device__ __forceinline__ void row_axpy(double* dst, const double* x, double alpha, const double* y, int n, int lane)
 {
     ROW4(n, lane, i) {

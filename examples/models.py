@@ -139,10 +139,12 @@ def cartpole_rk3_implicit(y, x, u, w):
     return y - cartpole_rk3_explicit(x, u, w)
 
 
-def build_cartpole(api, T=101, evaluate_hessian=True, parameterized=True):
+def build_cartpole(api, T=101, evaluate_hessian=True, parameterized=True, u_bnd=3.0):
     """`parameterized=True` is BASELINE config 2: start/goal enter through an 8-vector of
     per-problem parameters w = [x1; xT] seen by every knot (SURVEY Q10); False is the
-    example verbatim (constants captured in the closures)."""
+    example verbatim (constants captured in the closures). `u_bnd`: |u| <= u_bnd as the example's
+    Bound(action_lower, action_upper); None leaves the controls free (equality constraints only). Bounds
+    live on the host: the model library is the same."""
     n, m = 4, 1
     nw = 8 if parameterized else 0
     x1 = np.array([0.0, 0.0, 0.0, 0.0])
@@ -161,8 +163,7 @@ def build_cartpole(api, T=101, evaluate_hessian=True, parameterized=True):
         cT = lambda x, u, w: x - xT
     ct = api.Cost(ot, n, m, num_parameter=nw, evaluate_hessian=evaluate_hessian)
     cTc = api.Cost(oT, n, 0, num_parameter=nw, evaluate_hessian=evaluate_hessian)
-    u_bnd = 3.0
-    bndt = api.Bound(n, m, action_lower=[-u_bnd], action_upper=[u_bnd])
+    bndt = api.Bound(n, m) if u_bnd is None else api.Bound(n, m, action_lower=[-u_bnd], action_upper=[u_bnd])
     con1 = api.Constraint(c1, n, m, num_parameter=nw, evaluate_hessian=evaluate_hessian)
     conT = api.Constraint(cT, n, 0, num_parameter=nw, evaluate_hessian=evaluate_hessian)
     return dict(
