@@ -144,6 +144,7 @@ def lib() -> C.CDLL:
         "dto_kkt_resolve": (C.c_int, [vp, vp, i64]),
         "dto_sqp_default_options": (None, [C.POINTER(SqpOptions)]),
         "dto_sqp_solve": (C.c_int, [vp, C.POINTER(SqpOptions)] + [vp] * 12),
+        "dto_sqp_solve_ex": (C.c_int, [vp, C.POINTER(SqpOptions)] + [vp] * 4 + [i64] + [vp] * 8),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)

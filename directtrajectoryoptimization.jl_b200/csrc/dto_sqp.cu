@@ -536,17 +536,22 @@ __device__ __forceinline__ double wmaxnan(double m)
         m = (x__ > m || x__ != x__) ? x__ : m; \
     } while (0)
 
+// The five k_ip_* kernels read the bound values of problem b at lo + b * bstride, up + b * bstride. PP (per-problem bound
+// values, bstride = N_z) is a template flag so that the shared-bounds instantiation (bstride = 0) is the code without a stride.
+
 // after the callbacks (g, c, J, H at z): diagonal of K, barrier gradient into g, shifted constraint right-hand side,
 // residual of c(z) + t = 0 into ckeep, barrier value; first iteration: slacks and their multipliers
+template <bool PP>
 __global__ void k_ip_prepare(const dto_sqp_args a)
 {
     WARP_PROBLEM();
     const double mu = a.mu[b];
     double accB = 0.0, accI = 0.0;
     const double* z = a.z + b * a.N_z;
+    const double *lo = PP ? a.lo + b * a.bstride : a.lo, *up = PP ? a.up + b * a.bstride : a.up;
     for (int i = lane; i < a.N_z; i += 32) {
         const double hl = a.hasL[i], hu = a.hasU[i];
-        const double sL = hl > 0.0 ? z[i] - a.lo[i] : 1.0, sU = hu > 0.0 ? a.up[i] - z[i] : 1.0;
+        const double sL = hl > 0.0 ? z[i] - lo[i] : 1.0, sU = hu > 0.0 ? up[i] - z[i] : 1.0;
         a.diag[b * a.dim + i] = hl * a.zL[b * a.N_z + i] / sL + hu * a.zU[b * a.N_z + i] / sU;
         a.bg_w[b * a.N_z + i] += mu * (hu / sU - hl / sL);
         accB += hl * log(sL) + hu * log(sU);
@@ -576,16 +581,18 @@ __global__ void k_ip_prepare(const dto_sqp_args a)
     if (lane == 0) a.fbar[b] = -mu * accI - mu * accB;
 }
 
+template <bool PP>
 __global__ void k_ip_after_first(const dto_sqp_args a)
 {
     WARP_PROBLEM();
     const double mu = a.mu[b];
     const double* z = a.z + b * a.N_z;
     const double* rz = a.rhs + b * a.dim;
+    const double *lo = PP ? a.lo + b * a.bstride : a.lo, *up = PP ? a.up + b * a.bstride : a.up;
     double dr = 0.0, comp = 0.0, emu = 0.0;
     for (int i = lane; i < a.N_z; i += 32) {
         const double hl = a.hasL[i], hu = a.hasU[i];
-        const double sL = hl > 0.0 ? z[i] - a.lo[i] : 1.0, sU = hu > 0.0 ? a.up[i] - z[i] : 1.0;
+        const double sL = hl > 0.0 ? z[i] - lo[i] : 1.0, sU = hu > 0.0 ? up[i] - z[i] : 1.0;
         const double zL = a.zL[b * a.N_z + i], zU = a.zU[b * a.N_z + i];
         const double gshift = mu * (hu / sU - hl / sL);
         KEEPMAX(dr, (rz[i] - gshift - zL + zU) * a.free[i]);     // g + J'lam - z_L + z_U of the ORIGINAL problem
@@ -635,6 +642,7 @@ __global__ void k_ip_after_first(const dto_sqp_args a)
     }
 }
 
+template <bool PP>
 __global__ void k_ip_direction(const dto_sqp_args a)
 {
     WARP_PROBLEM();
@@ -642,6 +650,7 @@ __global__ void k_ip_direction(const dto_sqp_args a)
     const double tau = fmax(a.p.tau_min, 1.0 - mu);
     const double* sol = a.sol + b * a.dim;
     const double* z = a.z + b * a.N_z;
+    const double *lo = PP ? a.lo + b * a.bstride : a.lo, *up = PP ? a.up + b * a.bstride : a.up;
     const double big = 1.0e300;
     double gd = 0.0, c1 = 0.0, cl = 0.0, gdt = 0.0, amax = big, az = big;
     for (int i = lane; i < a.N_z; i += 32) {
@@ -649,7 +658,7 @@ __global__ void k_ip_direction(const dto_sqp_args a)
         a.dz[b * a.N_z + i] = d;
         gd += a.bg[b * a.N_z + i] * d;
         const double hl = a.hasL[i], hu = a.hasU[i];
-        const double sL = hl > 0.0 ? z[i] - a.lo[i] : 1.0, sU = hu > 0.0 ? a.up[i] - z[i] : 1.0;
+        const double sL = hl > 0.0 ? z[i] - lo[i] : 1.0, sU = hu > 0.0 ? up[i] - z[i] : 1.0;
         const double zL = a.zL[b * a.N_z + i], zU = a.zU[b * a.N_z + i];
         const double dzL = hl * (mu / sL - zL - (hl * zL / sL) * d);
         const double dzU = hu * (mu / sU - zU + (hu * zU / sU) * d);
@@ -704,6 +713,7 @@ __global__ void k_ip_direction(const dto_sqp_args a)
     }
 }
 
+template <bool PP>
 __global__ void k_ip_ls_round(const dto_sqp_args a, int32_t round)
 {
     WARP_PROBLEM();
@@ -711,10 +721,11 @@ __global__ void k_ip_ls_round(const dto_sqp_args a, int32_t round)
     double alpha = a.alpha[b];
     const double az = a.a_z[b];
     const double* bz = a.bz + b * a.N_z;
+    const double *lo = PP ? a.lo + b * a.bstride : a.lo, *up = PP ? a.up + b * a.bstride : a.up;
     double barB = 0.0, barI = 0.0, ct1 = 0.0, mdz = 0.0, mz = 0.0;
     for (int i = lane; i < a.N_z; i += 32) {
         const double hl = a.hasL[i], hu = a.hasU[i];
-        const double sL = hl > 0.0 ? fmax(bz[i] - a.lo[i], 1.0e-300) : 1.0, sU = hu > 0.0 ? fmax(a.up[i] - bz[i], 1.0e-300) : 1.0;
+        const double sL = hl > 0.0 ? fmax(bz[i] - lo[i], 1.0e-300) : 1.0, sU = hu > 0.0 ? fmax(up[i] - bz[i], 1.0e-300) : 1.0;
         barB += hl * log(sL) + hu * log(sU);
         KEEPMAX(mdz, a.dz[b * a.N_z + i]);
         KEEPMAX(mz, a.z[b * a.N_z + i]);
@@ -764,6 +775,7 @@ __global__ void k_ip_ls_round(const dto_sqp_args a, int32_t round)
     }
 }
 
+template <bool PP>
 __global__ void k_ip_end(const dto_sqp_args a)
 {
     WARP_PROBLEM();
@@ -776,10 +788,11 @@ __global__ void k_ip_end(const dto_sqp_args a)
             for (int j = lane; j < a.N_c; j += 32) a.lam[b * a.N_c + j] *= (a.p.any_ineq ? a.hasI[j] : 0.0);
     }
     const double ks = a.p.kappa_sigma;
+    const double *lo = PP ? a.lo + b * a.bstride : a.lo, *up = PP ? a.up + b * a.bstride : a.up;
     for (int i = lane; i < a.N_z; i += 32) {      // z_L, z_U within [mu / (kappa s), kappa mu / s] of the new slacks
         const double hl = a.hasL[i], hu = a.hasU[i];
         const double zi = a.z[b * a.N_z + i];
-        const double sL = hl > 0.0 ? zi - a.lo[i] : 1.0, sU = hu > 0.0 ? a.up[i] - zi : 1.0;
+        const double sL = hl > 0.0 ? zi - lo[i] : 1.0, sU = hu > 0.0 ? up[i] - zi : 1.0;
         a.zL[b * a.N_z + i] = hl * fmax(fmin(a.zL[b * a.N_z + i], ks * mu / sL), mu / (ks * sL));
         a.zU[b * a.N_z + i] = hu * fmax(fmin(a.zU[b * a.N_z + i], ks * mu / sU), mu / (ks * sU));
     }
@@ -1068,11 +1081,14 @@ extern "C" int dto_sqp_k_reg_pick(const dto_sqp_args* a, int32_t count, int32_t 
     const cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? 0 : -(int)e;
 }
-extern "C" int dto_sqp_k_ip_prepare(const dto_sqp_args* a, void* s) { return launch_warp_per(k_ip_prepare, a->B, s, *a); }
-extern "C" int dto_sqp_k_ip_after_first(const dto_sqp_args* a, void* s) { return launch_warp_per(k_ip_after_first, a->B, s, *a); }
-extern "C" int dto_sqp_k_ip_direction(const dto_sqp_args* a, void* s) { return launch_warp_per(k_ip_direction, a->B, s, *a); }
-extern "C" int dto_sqp_k_ip_ls_round(const dto_sqp_args* a, int32_t round, void* s) { return launch_warp_per(k_ip_ls_round, a->B, s, *a, round); }
-extern "C" int dto_sqp_k_ip_end(const dto_sqp_args* a, void* s) { return launch_warp_per(k_ip_end, a->B, s, *a); }
+extern "C" int dto_sqp_k_ip_prepare(const dto_sqp_args* a, void* s) { return launch_warp_per(a->bstride ? k_ip_prepare<true> : k_ip_prepare<false>, a->B, s, *a); }
+extern "C" int dto_sqp_k_ip_after_first(const dto_sqp_args* a, void* s) { return launch_warp_per(a->bstride ? k_ip_after_first<true> : k_ip_after_first<false>, a->B, s, *a); }
+extern "C" int dto_sqp_k_ip_direction(const dto_sqp_args* a, void* s) { return launch_warp_per(a->bstride ? k_ip_direction<true> : k_ip_direction<false>, a->B, s, *a); }
+extern "C" int dto_sqp_k_ip_ls_round(const dto_sqp_args* a, int32_t round, void* s)
+{
+    return launch_warp_per(a->bstride ? k_ip_ls_round<true> : k_ip_ls_round<false>, a->B, s, *a, round);
+}
+extern "C" int dto_sqp_k_ip_end(const dto_sqp_args* a, void* s) { return launch_warp_per(a->bstride ? k_ip_end<true> : k_ip_end<false>, a->B, s, *a); }
 extern "C" int dto_sqp_k_qn_update(const dto_sqp_args* a, void* s)
 {
     const int64_t threads = a->B * a->T * a->qn_W;

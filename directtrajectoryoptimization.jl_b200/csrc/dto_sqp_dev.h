@@ -68,7 +68,9 @@ typedef struct dto_sqp_args {
     int32_t* tries;       /* [B] inertia-correction tries used by the problem in this iteration */
     int32_t* alist;       /* [B] problems that have not converged (written by the first check, for the next iteration) */
     /* interior-point mode */
-    const double *hasL, *hasU, *lo, *up;   /* [N_z] 0/1 masks and finite bound values (0 where absent)        */
+    const double *hasL, *hasU;             /* [N_z] 0/1 masks (one bound pattern per batch)                     */
+    const double *lo, *up;                 /* finite bound values (0 where absent): problem b's at lo + b * bstride */
+    int64_t bstride;                       /* 0: one [N_z] pair for every problem; N_z: [B][N_z]                  */
     const double* hasI;                    /* [N_c] 1 = inequality row c_i(z) <= 0                              */
     double *zL, *zU, *dzL, *dzU;           /* [B][N_z] bound multipliers and their steps                        */
     double *t, *dt;                        /* [B][N_c] slacks of the inequality rows and their steps            */

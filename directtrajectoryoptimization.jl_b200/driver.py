@@ -166,7 +166,10 @@ def solve_batch(nlp, z0: np.ndarray, options: Optional[dict] = None, record_iter
     else:
         hr = hc = np.ones(0, dtype=np.int64)
     structures = ((jr - 1, jc - 1), (hr - 1, hc - 1), nlp.num_variables, nlp.num_constraint, use_hessian)
-    bounds = (nlp.variable_bounds, nlp.constraint_bounds)
+    # every problem's own variable bounds: [B, N_z] rows when the batch has per-problem values, else the shared pair
+    lo, up = (np.asarray(v, dtype=np.float64) for v in getattr(nlp, "batch_variable_bounds", nlp.variable_bounds))
+    cbounds = nlp.constraint_bounds
+    bounds_of = (lambda b: ((lo[b], up[b]), cbounds)) if lo.ndim == 2 else (lambda b: ((lo, up), cbounds))
     opts = {"gtol": 1e-8, "xtol": 1e-10, "maxiter": 1000, "verbose": 0}
     opts.update(options or {})
     z0 = np.asarray(z0, dtype=np.float64).reshape(B, nlp.num_variables)
@@ -177,7 +180,7 @@ def solve_batch(nlp, z0: np.ndarray, options: Optional[dict] = None, record_iter
 
     def run(b):
         try:
-            results[b] = task(broker, b, z0[b].copy(), structures, bounds, opts, iterates[b] if iterates is not None else None)
+            results[b] = task(broker, b, z0[b].copy(), structures, bounds_of(b), opts, iterates[b] if iterates is not None else None)
         except BaseException as e:  # noqa: BLE001
             errors[b] = e
 

@@ -111,6 +111,7 @@ class BatchedNLPData:
         self.num_parameter = int(L.dto_num_parameter(h))
         self._batch = None
         self._bounds = bounds
+        self._bounds_host = None        # [lower, upper] of set_variable_bounds, [B, N_z] each
 
     # ---- structure (host only)
     def jacobian_structure_arrays(self):
@@ -185,11 +186,15 @@ class BatchedNLPData:
 
     @property
     def variable_bounds(self):
-        """primal_bounds (src/data.jl:123-133)."""
+        """primal_bounds (src/data.jl:123-133) of the Bound objects the batch was built with."""
+        return self.primal_bounds(self._bounds)
+
+    def primal_bounds(self, bounds):
+        """[lower, upper] ([N_z] each) of a list of T Bound objects, laid out as primal_bounds (src/data.jl:123-133)."""
         lo = np.full(self.num_variables, -np.inf)
         hi = np.full(self.num_variables, np.inf)
         xs, nx, us, nu = self.knot_layout()
-        for t, b in enumerate(self._bounds or []):
+        for t, b in enumerate(bounds or []):
             if len(b.state_lower) > 0:
                 lo[xs[t] - 1: xs[t] - 1 + nx[t]] = b.state_lower
             if len(b.state_upper) > 0:
@@ -199,6 +204,29 @@ class BatchedNLPData:
             if len(b.action_upper) > 0:
                 hi[us[t] - 1: us[t] - 1 + nu[t]] = b.action_upper
         return [lo, hi]
+
+    def set_variable_bounds(self, lower, upper):
+        """Bound values per problem: lower, upper [B, N_z] (row b = problem b's primal_bounds), or None for both to return to
+        the Bound objects. The solvers take one bound pattern per batch -- which variables are pinned (lower == upper), which
+        have a finite lower and which a finite upper bound -- and every problem's own values; a batch whose rows differ in
+        pattern is refused when it is solved. Kept on the host (a solve over several devices hands every shard its rows)."""
+        if lower is None and upper is None:
+            self._bounds_host = None
+            return
+        if lower is None or upper is None:
+            raise ValueError("set_variable_bounds: lower and upper come together (or both None)")
+        shape = (self.batch, self.num_variables)
+        lo = np.array(_f64(lower, shape, "lower"), dtype=np.float64, copy=True).reshape(shape)
+        up = np.array(_f64(upper, shape, "upper"), dtype=np.float64, copy=True).reshape(shape)
+        self._bounds_host = [lo, up]
+
+    @property
+    def batch_variable_bounds(self):
+        """[lower, upper] as the solvers take them: the [B, N_z] rows of set_variable_bounds, or else the shared [N_z] pair
+        of `variable_bounds`."""
+        if self._bounds_host is not None:
+            return [self._bounds_host[0], self._bounds_host[1]]
+        return self.variable_bounds
 
     # ---- device batch
     @property
@@ -298,6 +326,8 @@ class BatchedNLPData:
         other.__dict__.update(self.__dict__)
         other._batch = None
         other.batch = int(batch) if batch is not None else self.batch
+        if other.batch != self.batch:       # per-problem rows belong to this batch's problems: the caller hands over a slice
+            other._bounds_host = None
         other.devices = list(devices) if devices is not None else self.devices
         return other
 
@@ -420,6 +450,18 @@ class Solver:
         rows = slice(None) if problem is None else problem
         for t, xt in enumerate(states):
             self._initial[rows, xs[t] - 1: xs[t] - 1 + len(xt)] = np.asarray(xt, float)
+
+    def set_bounds(self, bounds: List[Bound], problem: Optional[int] = None):
+        """The variable bounds of one problem (or, with problem=None, of every problem): a list of T Bound objects laid out
+        exactly as the `bounds` argument (primal_bounds, src/data.jl:123-133). Problems of one batch may differ in bound
+        values -- start and end states pinned by Bound(state_lower = x1, state_upper = x1), actuator limits -- but not in
+        pattern (which variables are pinned, lower-bounded, upper-bounded): see BatchedNLPData.set_variable_bounds."""
+        lo, up = self.nlp.primal_bounds(bounds)
+        if self.nlp._bounds_host is None:       # the first per-problem row: every problem starts from the Bound objects
+            self.nlp.set_variable_bounds(*(np.tile(v, (self.nlp.batch, 1)) for v in self.nlp.variable_bounds))
+        sel = slice(None) if problem is None else problem
+        self.nlp._bounds_host[0][sel] = lo      # (in place: a batch of thousands is filled one problem at a time)
+        self.nlp._bounds_host[1][sel] = up
 
     def initialize_controls(self, actions, problem: Optional[int] = None):
         _, _, us, _ = self.nlp.knot_layout()

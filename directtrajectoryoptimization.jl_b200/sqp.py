@@ -494,10 +494,26 @@ def chain_from_elements(elements, blocks):
 def bound_arrays(lo, up, options: Optional[SQPOptions] = None, clo=None, cup=None, scale: float = 1.0):
     """numpy: primal_bounds (src/data.jl:123-133) -> what `solve` needs. Returns (fixed, bounds): `fixed` = variables pinned
     by lo == up; `bounds` = None when no other finite bound exists, else dict(hasL, hasU, lo, up, pushL, pushU) with 0/1
-    masks, finite values (0 where absent) and the distances the starting point is pushed inside (Ipopt's bound_push/frac)."""
+    masks, finite values (0 where absent) and the distances the starting point is pushed inside (Ipopt's bound_push/frac).
+    lo, up may be [N_z] (every problem) or [B, N_z] (row b = problem b's values): `fixed`, hasL and hasU are then still [N_z]
+    -- one bound pattern per batch, checked to be common to all rows (ValueError otherwise) -- and lo, up, pushL, pushU are
+    [B, N_z], each row computed by the same elementwise operations as the [N_z] case (the same values, bit for bit)."""
     import numpy as np
     o = options or SQPOptions()
     lo, up = np.asarray(lo, float), np.asarray(up, float)
+    rows = lo.ndim == 2
+    if rows:
+        bad = np.isnan(lo) | np.isnan(up) | (np.isfinite(lo) & np.isfinite(up) & (lo > up))
+        if bad.any():
+            p, i = (int(v[0]) for v in np.nonzero(bad))
+            raise ValueError(f"problem {p}, variable index {i}: bounds [{lo[p, i]}, {up[p, i]}]")
+        fx = np.isfinite(lo) & (lo == up)
+        for name, pat in (("pinned", fx), ("lower-bounded", np.isfinite(lo) & ~fx), ("upper-bounded", np.isfinite(up) & ~fx)):
+            diff = pat != pat[:1]
+            if diff.any():
+                p, i = (int(v[0]) for v in np.nonzero(diff))
+                raise ValueError(f"problem {p}, variable index {i}: bounds [{lo[p, i]}, {up[p, i]}] differ from problem 0's "
+                                 f"[{lo[0, i]}, {up[0, i]}] in which variables are {name}: a batch has one bound pattern")
     fixed = np.isfinite(lo) & (lo == up)
     if scale != 1.0:        # continuation stage: two-sided bounds widened about their midpoint (one-sided and pinned ones stay)
         two = np.isfinite(lo) & np.isfinite(up) & ~fixed
@@ -512,13 +528,15 @@ def bound_arrays(lo, up, options: Optional[SQPOptions] = None, clo=None, cup=Non
     if hasI.any() and not (np.all(np.isneginf(np.asarray(clo, float)[hasI])) and np.all(np.asarray(cup, float)[hasI] == 0.0)):
         raise NotImplementedError("sqp: inequality rows other than c(z) <= 0 are outside this solver's scope")
     if not (hasL.any() or hasU.any() or hasI.any()):
-        return fixed, None
+        return (fixed[0] if rows else fixed), None
     if np.any((hasL & hasU) & (lo >= up)):
         raise ValueError("a variable's lower bound exceeds its upper bound")
     l0, u0 = np.where(hasL, lo, 0.0), np.where(hasU, up, 0.0)
     width = np.where(hasL & hasU, u0 - l0, np.inf)
     pushL = np.where(hasL, np.minimum(o.bound_push * np.maximum(1.0, np.abs(l0)), o.bound_frac * width), 0.0)
     pushU = np.where(hasU, np.minimum(o.bound_push * np.maximum(1.0, np.abs(u0)), o.bound_frac * width), 0.0)
+    if rows:        # the pattern is the batch's (checked above): one mask per variable
+        fixed, hasL, hasU = fixed[0], hasL[0], hasU[0]
     return fixed, dict(hasL=hasL.astype(np.float64), hasU=hasU.astype(np.float64), lo=l0, up=u0, pushL=pushL, pushU=pushU,
                        hasI=hasI.astype(np.float64))
 
@@ -674,7 +692,7 @@ class DeviceBackend:
         dev = torch.device("cuda", nlp.shard_device(0))
         self.xp = _XP(torch, dev)
         self.B, self.N_z, self.N_c = nlp.batch, nlp.num_variables, nlp.num_constraint
-        lo, up = nlp.variable_bounds
+        lo, up = nlp.batch_variable_bounds       # [N_z] each, or [B, N_z]: every problem's values (one pattern)
         import numpy as np
         clo, cup = nlp.constraint_bounds
         # Bound(state_lower = x1, state_upper = x1): pinned variables; any other finite bound: interior point in `solve`
@@ -736,6 +754,10 @@ class DeviceBackend:
         idx = keep.nonzero().flatten()
         n = int(idx.numel())
         nlp2 = self.nlp.new_batch(batch=n)
+        rows = self.nlp._bounds_host
+        if rows is not None:
+            sel = idx.cpu().numpy()
+            nlp2.set_variable_bounds(rows[0][sel], rows[1][sel])
         dev = self.xp.device
         if self.nlp.num_parameter:
             nw = self.nlp.num_parameter
@@ -920,14 +942,15 @@ def solve_native(nlp, z0, lam0=None, options: Optional[SQPOptions] = None) -> SQ
         lam0 = np.ascontiguousarray(lam0, dtype=np.float64)
         if lam0.shape != (B, N_c):
             raise ValueError(f"lam0 has shape {lam0.shape}, expected {(B, N_c)}")
-    lo, up = (np.ascontiguousarray(v, dtype=np.float64) for v in nlp.variable_bounds)
+    lo, up = (np.ascontiguousarray(v, dtype=np.float64) for v in nlp.batch_variable_bounds)
+    stride = N_z if lo.ndim == 2 else 0         # [B, N_z]: one row per problem (dto_sqp_solve_ex); [N_z]: shared by all
     z, lam = np.empty((B, N_z)), np.empty((B, N_c))
     iters, done = np.empty(B, np.int32), np.empty(B, np.uint8)
     cv, dr, f = np.empty(B), np.empty(B), np.empty(B)
     stats = np.zeros(16, np.int64)
     ptr = lambda a: None if a is None else a.ctypes.data  # noqa: E731
-    _lib.check(L.dto_sqp_solve(nlp.handle, C.byref(co), ptr(z0), ptr(lam0), ptr(lo), ptr(up), ptr(z), ptr(lam), ptr(iters), ptr(done),
-                               ptr(cv), ptr(dr), ptr(f), ptr(stats)))
+    _lib.check(L.dto_sqp_solve_ex(nlp.handle, C.byref(co), ptr(z0), ptr(lam0), ptr(lo), ptr(up), stride, ptr(z), ptr(lam), ptr(iters),
+                                  ptr(done), ptr(cv), ptr(dr), ptr(f), ptr(stats)))
     res = SQPResult(z, lam, iters.astype(np.float64), done.astype(bool), cv, dr, f, [])
     res.staged = done == 2          # converged by the bound continuation (see solve_bounded)
     res.stats = dict(iterations=int(stats[0]), launches=int(stats[1]), factorisations=int(stats[2]), syncs=int(stats[3]),
@@ -941,7 +964,7 @@ def solve_native(nlp, z0, lam0=None, options: Optional[SQPOptions] = None) -> SQ
 def solve_native_sharded(nlp, z0, lam0=None, options: Optional[SQPOptions] = None) -> SQPResult:
     """`solve_native` for a batch spread over several devices (row (e): problems are independent, contiguous shards, no
     collective): dto_sqp_solve drives ONE device, so every shard gets its own one-device batch of the same shape (model library
-    and static tables shared, its slice of the per-problem parameters), the solves run side by side from one host thread each
+    and static tables shared, its slice of the per-problem parameters and bounds), the solves run side by side from one host thread each
     (ctypes releases the GIL for the duration of the C call), and the results are put back in the caller's order; the final
     iterate also becomes the resident z of the original batch (get_trajectory)."""
     import threading
@@ -953,6 +976,7 @@ def solve_native_sharded(nlp, z0, lam0=None, options: Optional[SQPOptions] = Non
     w = getattr(nlp, "_w_host", None)
     if nlp.num_parameter and w is None:
         raise RuntimeError("solve_native_sharded: the per-problem parameters were not set through set_parameters")
+    rows = getattr(nlp, "_bounds_host", None)
     results, errors = [None] * len(parts), []
 
     def work(k, device, begin, size):
@@ -963,6 +987,8 @@ def solve_native_sharded(nlp, z0, lam0=None, options: Optional[SQPOptions] = Non
             sub = nlp.new_batch(batch=size, devices=[device])
             if nlp.num_parameter:
                 sub.set_parameters(w[begin:begin + size])
+            if rows is not None:
+                sub.set_variable_bounds(rows[0][begin:begin + size], rows[1][begin:begin + size])
             results[k] = solve_native(sub, z0[begin:begin + size], None if lam0 is None else lam0[begin:begin + size], options)
         except Exception as e:  # noqa: BLE001 - re-raised in the caller's thread
             errors.append(e)

@@ -327,6 +327,16 @@ void dto_sqp_default_options(dto_sqp_options* o);
 int dto_sqp_solve(dto_batch* b, const dto_sqp_options* options, const double* z0, const double* lambda0, const double* lower,
                   const double* upper, double* z, double* lambda, int32_t* iterations, uint8_t* converged,
                   double* constraint_violation, double* dual_residual, double* objective, int64_t* stats);
+/* dto_sqp_solve with bound values per problem: problem p's bounds are lower + p * bounds_stride and upper + p * bounds_stride.
+ * bounds_stride = 0: one [N_z] pair for every problem (= dto_sqp_solve); bounds_stride = N_z: [B][N_z], problem-major like z0;
+ * any other value -> DTO_ERR_BAD_ARG. A batch has ONE bound pattern -- which variables are pinned (lower == upper), which have a
+ * finite lower bound, which a finite upper bound -- and each problem its own values: pinned values, bound values, the starting
+ * point's push inside them and the continuation's widening about the problem's own midpoints. Every problem is checked: NaN or
+ * lower > upper -> DTO_ERR_BAD_ARG; a pattern that differs from problem 0's -> DTO_ERR_UNSUPPORTED (the KKT ordering of pinned
+ * variables and the interior-point masks are per shape); both messages name the problem and the variable. */
+int dto_sqp_solve_ex(dto_batch* b, const dto_sqp_options* options, const double* z0, const double* lambda0, const double* lower,
+                     const double* upper, int64_t bounds_stride, double* z, double* lambda, int32_t* iterations, uint8_t* converged,
+                     double* constraint_violation, double* dual_residual, double* objective, int64_t* stats);
 
 #ifdef __cplusplus
 }

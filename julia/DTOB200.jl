@@ -408,7 +408,9 @@ end
 
 All problems of a one-device batch from the guesses `z0[n, B]` (column b = problem b), in lock step on the GPU: the role
 Ipopt plays for one problem in `solve!(solver)` (src/solver.jl:45-47). Equality rows and rows c(z) <= 0; variables free, pinned
-by `lower[i] == upper[i]`, or bounded (interior point). Returns a named tuple
+by `lower[i] == upper[i]`, or bounded (interior point). `lower` and `upper` are vectors of length n (every problem) or
+`n × B` matrices (column b = problem b's bounds, e.g. its own pinned start state or actuator limits); the columns must share one
+bound pattern (which variables are pinned, lower-bounded, upper-bounded). Returns a named tuple
 `(z, lambda, iterations, converged, constraint_violation, dual_residual, objective, stats)`.
 """
 function solve_batch(nlp::BatchedNLPData, z0::Matrix{Float64}; lower=nothing, upper=nothing, options::SQPOptions=SQPOptions(), lambda0=nothing)
@@ -419,14 +421,20 @@ function solve_batch(nlp::BatchedNLPData, z0::Matrix{Float64}; lower=nothing, up
     its, conv = Vector{Int32}(undef, B), Vector{UInt8}(undef, B)
     cv, dr, f = Vector{Float64}(undef, B), Vector{Float64}(undef, B), Vector{Float64}(undef, B)
     stats = zeros(Int64, 16)
+    (lower === nothing) == (upper === nothing) || throw(ArgumentError("lower and upper come together"))
+    stride = 0                                                 # vectors: one pair for every problem
+    if lower !== nothing && lower isa AbstractMatrix
+        size(lower) == (n, B) && size(upper) == (n, B) || throw(DimensionMismatch("lower and upper must be [num_variables, batch] matrices"))
+        stride = n                                             # column b = problem b (the ABI's [B][N_z])
+    end
     lo = lower === nothing ? Ptr{Float64}(C_NULL) : pointer(lower)
     up = upper === nothing ? Ptr{Float64}(C_NULL) : pointer(upper)
     l0 = lambda0 === nothing ? Ptr{Float64}(C_NULL) : pointer(lambda0)
     GC.@preserve lower upper lambda0 begin
-        check(ccall((:dto_sqp_solve, libdto), Cint,
-                    (Ptr{Cvoid}, Ref{SQPOptions}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+        check(ccall((:dto_sqp_solve_ex, libdto), Cint,
+                    (Ptr{Cvoid}, Ref{SQPOptions}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Float64}, Ptr{Float64},
                      Ptr{Int32}, Ptr{UInt8}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}),
-                    nlp.batch, Ref(options), z0, l0, lo, up, z, lam, its, conv, cv, dr, f, stats))
+                    nlp.batch, Ref(options), z0, l0, lo, up, stride, z, lam, its, conv, cv, dr, f, stats))
     end
     (z=z, lambda=lam, iterations=Int.(its), converged=conv .!= 0, constraint_violation=cv, dual_residual=dr, objective=f, stats=stats)
 end
